@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- self-play moves/sec (8x8, 800 sims) on N B200s, plus env steps/sec (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[2] -- 8x8 board, default 128x10 network with the
@@ -226,6 +226,55 @@ def tensor_roofline(peaks, evals, prof, ms, flops_leaf, extra=None):
     return roof
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(engine, eng, plies, out_dir):
+    """Writes the replay records (Engine.replay_window: board before the move, root visit counts, game serial, ply, player)
+    that the timed self-play holds after its last step, with the result code of each record's game from the results
+    table, as float32 / float64 .npy files under out_dir, sorted by (game serial, ply).
+
+    The records kept are those of the games the reset starts (serials 0 .. n_games - 1) at plies 0 .. plies - 1, so that
+    runs with the same arguments write the same records.  That set does not depend on timing: a search needs at most
+    SIMS + 1 evaluation steps and a finished search moves in the same step, so after L launches of SIMS + 1 steps every
+    slot has made at least L moves (the caller passes L - 1); the content of a record depends only on the seed, the game
+    serial and the ply.  Which records a given launch appends does depend on timing: simulations that end in revisited
+    terminals are advanced by background warps while the tower runs.  For the same reason a game that goes on past the
+    kept plies may or may not be over when the run stops, so its result code is written as 0 (not over by the last kept
+    ply); only games that end within the kept plies carry their code.  Above DUMP_BYTES a fixed, seeded sample is written."""
+    import numpy as np
+    from yinyang_game_alphazero_b200 import bitboard
+    n = eng.stats().examples
+    if n > eng.replay_capacity:
+        raise RuntimeError(f"replay ring wrapped ({n} records, capacity {eng.replay_capacity}): the first games are gone")
+    rec = eng.replay_window(0, n)
+    results = engine._to_host(eng.replay_views()["results"])[0]
+    serial, ply = rec["game_serial"].astype(np.int64), rec["ply"].astype(np.int64)
+    keep = np.flatnonzero((serial >= 0) & (serial < eng.n_games) & (ply < plies))
+    keep = keep[np.lexsort((ply[keep], serial[keep]))]
+    code = results[serial % len(results)]
+    per_game = np.bincount(serial[keep], minlength=eng.n_games)
+    short = np.flatnonzero(per_game != plies)
+    if len(np.unique(serial[keep] * plies + ply[keep])) != len(keep) or np.any(code[keep][np.isin(serial[keep], short)] == 0) \
+            or np.any(per_game[short] == 0):
+        raise RuntimeError(f"the first {eng.n_games} games do not all hold plies 0..{plies - 1} (or their whole game)")
+    first = (serial >= 0) & (serial < eng.n_games)
+    ended_within = np.bincount(serial[first], minlength=eng.n_games) <= plies     # every move of the game is a kept record
+    code = np.where(first & ended_within[np.where(first, serial, 0)], code, 0)
+    out = {"boards": bitboard.unpack_boards(rec["black"], rec["white"], ROWS, COLS).astype(np.float32),
+           "visit_counts": rec["counts"].astype(np.float32),
+           "game_serial": serial.astype(np.float64),
+           "ply": ply.astype(np.float32),
+           "player": rec["player"].astype(np.float32),
+           "game_result": code.astype(np.float32)}
+    per_record = sum(a[0].nbytes for a in out.values())
+    if len(keep) * per_record > DUMP_BYTES:
+        keep = keep[np.sort(np.random.default_rng(0).choice(len(keep), DUMP_BYTES // per_record, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[keep])
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -265,6 +314,8 @@ def run_b200(args):
     clocks = sampler.stop()
     launches = engine._lib.lib().yy_launch_count() - launches1 - 2 * args.warmup
     value = moves / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(engine, eng, max(1, args.warmup + args.steps - 1), args.dump_outputs)
 
     # replay gather (north star: gather replay samples over NCCL), outside the timed region
     t_gather, n_records = (yyd.gather_replay_counts(eng) if world > 1 else (0.0, min(st.examples, eng.replay_capacity)))
@@ -785,7 +836,10 @@ def main():
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="developer runs: only the self-play legs (value, e2e, roofline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the replay records of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:
