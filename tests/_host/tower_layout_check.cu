@@ -53,3 +53,16 @@ extern "C" int yyh_tower_layout(int rows, int cols, int* out_layout, int* out_bo
   }
   return 0;
 }
+
+// The choices of the persistent kernel's code paths for a board, as yy_fused.cu makes them: out = layout, group size
+// before / after the FC_N clamp, tiles of a full group, policy M tiles, K panels, K stages per head, rows of the last
+// policy tile, boards per heads pass.  Returns -1 when the network kernel does not accept the board.
+extern "C" int yyh_tower_classes(int rows, int cols, int* out) {
+  if (!nn_geometry_ok(rows, cols)) return -1;
+  const TowerGeo raw = make_tower_geo(rows, cols, 10);
+  const TowerGeo g = make_fused_geo(rows, cols, 10);
+  const FcGeo f = make_fc_geo(g.A);
+  const int v[9] = {g.row_aligned, raw.Gb, g.Gb, tower_tiles_for(g, g.Gb), f.Tp, f.n_panels, f.KS, f.Rp_last, fused_batch_boards(g)};
+  for (int i = 0; i < 9; ++i) out[i] = v[i];
+  return 0;
+}

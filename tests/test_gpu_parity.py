@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 from conftest import golden_files, load_golden, random_play_boards, randomise_bn
+from exact_net import REPRESENTATIVES
 
 pytestmark = pytest.mark.gpu
 
@@ -247,7 +248,9 @@ def test_mcts_external_evaluator_seam(eng, oracle_mod):
 @pytest.mark.parametrize("cfg", [(8, 8, 128, 10, 300, False), (8, 8, 128, 10, 64, True), (8, 8, 128, 0, 40, True),
                                  (8, 8, 128, 1, 40, True), (6, 6, 128, 3, 64, True), (8, 8, 32, 2, 50, True),
                                  (16, 16, 128, 1, 9, True), (5, 7, 64, 2, 33, True), (8, 8, 128, 1, 37, True),
-                                 (16, 16, 64, 2, 35, False), (8, 8, 128, 2, 1000, False), (6, 6, 128, 1, 5000, True)])
+                                 (16, 16, 64, 2, 35, False), (8, 8, 128, 2, 1000, False), (6, 6, 128, 1, 5000, True)]
+                         # one board of every geometry class of the kernel (tests/exact_net.py REPRESENTATIVES)
+                         + [(n, m, C, min(b, 2), 40, True) for n, m, C, b in REPRESENTATIVES if (n, m) not in {(8, 8), (6, 6), (16, 16), (5, 7)}])
 def test_network_matches_fp32_reference(eng, oracle_mod, cfg):
     """bf16 tcgen05 tower + heads vs the fp32 torch network (reference semantics, neural_network.py:94-154).
     Stated tolerance (bf16 weights + bf16 inter-layer activations, fp32 accumulate), measured headroom ~2x:

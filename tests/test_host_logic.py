@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, golden_files, load_golden, randomise_bn
+from exact_net import REPRESENTATIVES
 
 
 def _host_rules(lib, bbm, boards, players, actions, n, m, flags=0, stub=False):
@@ -320,3 +321,54 @@ def test_tower_layouts_structural(host_tower_lib, shape, layout, useful):
     rc = host_tower_lib.yyh_tower_layout(n, m, ctypes.byref(lay), ctypes.byref(gb), ctypes.byref(T), ctypes.byref(u))
     assert rc == 0, rc
     assert lay.value == layout and u.value >= useful and gb.value * n * m <= 128 * T.value
+
+
+def test_tower_layouts_structural_all_geometries(host_tower_lib):
+    """The structural walk above for every board the network kernel accepts (n, m <= 32, n * m <= 256, cols + 2 <=
+    TW_PAD: 500 boards); the rules' other boards are refused for being too wide."""
+    lay, gb, T = ctypes.c_int(), ctypes.c_int(), ctypes.c_int()
+    u = ctypes.c_double()
+    ok = []
+    for n in range(1, 33):
+        for m in range(1, 33):
+            if n * m > 256:
+                continue
+            rc = host_tower_lib.yyh_tower_layout(n, m, ctypes.byref(lay), ctypes.byref(gb), ctypes.byref(T), ctypes.byref(u))
+            if rc == -1:
+                assert m + 2 > 24, (n, m)
+                continue
+            assert rc == 0, (n, m, rc)
+            assert gb.value * n * m <= 128 * T.value, (n, m)
+            ok.append((n, m))
+    assert len(ok) == 500
+
+
+def test_geometry_classes_have_gpu_representatives(host_tower_lib):
+    """Every code-path class of the network kernel (exact_net.geometry_class) over all accepted boards has a board in
+    the list the exact GPU tests run (exact_net.REPRESENTATIVES)."""
+    import exact_net as X
+    classes = {}
+    for g in X.supported_geometries(host_tower_lib):
+        classes.setdefault(X.geometry_class(X.tower_classes(host_tower_lib, *g)), []).append(g)
+    covered = {X.geometry_class(X.tower_classes(host_tower_lib, n, m)) for n, m, _, _ in X.REPRESENTATIVES}
+    missing = {k: v[:4] for k, v in classes.items() if k not in covered}
+    assert not missing, missing
+    layouts = {X.tower_classes(host_tower_lib, n, m)["layout"] for n, m, _, b in X.REPRESENTATIVES if b == 10}
+    assert layouts == {k[0] for k in classes}, "a 128 x 10 net for every position layout"
+
+
+@pytest.mark.parametrize("n,m,channels,blocks", REPRESENTATIVES)
+def test_exact_network_packs_and_emulates_bit_exact(yy, oracle_mod, n, m, channels, blocks):
+    """The integer networks of the exact GPU tests: the builder's invariants hold on the positions, the packer folds them
+    into exactly the intended weights (both conv streams, biases, FC stream and sections), and for shallow nets the numpy
+    emulation of the kernel's dataflow reproduces the float64 reference's logits bit for bit."""
+    import emulate_tower as emu
+    import exact_net as X
+    boards = X.positions(oracle_mod, n, m, 12, seed=n * 100 + m)
+    net = X.ExactNet(n, m, channels, blocks, seed=1000 + n * 100 + m, boards=boards)
+    assert np.array_equal(net.logits, np.round(net.logits)) and np.all(np.abs(net.logits) < 2 ** 24)
+    img, lay = X.check_packed_image(net)
+    if blocks <= 2:
+        lg, v, _ = emu.forward(img, lay, n, m, blocks, boards)
+        assert np.array_equal(lg, net.logits.astype(np.float32))
+        assert X.ulp_distance(v, np.tanh(net.pre_value).astype(np.float32)).max() <= 2

@@ -858,12 +858,6 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-static int fused_batch_boards(const TowerGeo& g) {
-  if (g.row_aligned == 4) return FC_N;   // groups of 12 boards: a heads pass takes 12 + 12 + 8 (the last group of a batch may be partial)
-  int per = (FC_N / g.Gb) * g.Gb;
-  return per > 0 ? per : g.Gb;
-}
-
 template <int NW, int CG>
 static int launch_fused(NNState& nn, const FusedArgs& fa, const EngineDev& dev, uint32_t rule_flags, int grid, cudaStream_t s) {
   static bool attr_set[8] = {};
@@ -896,8 +890,7 @@ int nn_fused_run(NNState& nn, const EngineDev* dev, uint32_t rule_flags, const u
   if (count > nn.max_boards) return set_error(YY_ERR_INVALID, "fused run: %lld boards exceed the head-feature scratch (%d)", (long long)count, nn.max_boards);
   if ((mode != YY_FUSED_FORWARD) != (dev != nullptr)) return set_error(YY_ERR_INVALID, "fused run: mode / engine state mismatch");
   FusedArgs fa{};
-  fa.g = make_tower_geo(nn.rows, nn.cols, nn.blocks);
-  if (fa.g.Gb > FC_N) fa.g.Gb = FC_N;
+  fa.g = make_fused_geo(nn.rows, nn.cols, nn.blocks);
   fa.fc = make_fc_geo(nn.A);
   if (use_nn) {
     const WeightLayout wl = weight_layout(nn.rows, nn.cols, nn.blocks);

@@ -245,5 +245,17 @@ inline TowerGeo make_tower_geo(int rows, int cols, int blocks) {
   return g;
 }
 
+// The persistent kernel's geometry: a group holds at most FC_N boards, so that a heads pass takes whole groups.
+inline TowerGeo make_fused_geo(int rows, int cols, int blocks) {
+  TowerGeo g = make_tower_geo(rows, cols, blocks);
+  if (g.Gb > FC_N) g.Gb = FC_N;
+  return g;
+}
+// boards per heads pass of the persistent kernel (whole groups, except possibly the last group of a batch)
+inline int fused_batch_boards(const TowerGeo& g) {
+  if (g.row_aligned == 4) return FC_N;   // groups of 12 boards: a heads pass takes 12 + 12 + 8 (the last group of a batch may be partial)
+  int per = (FC_N / g.Gb) * g.Gb;
+  return per > 0 ? per : g.Gb;
+}
 
 }  // namespace yy
