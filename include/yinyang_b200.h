@@ -120,6 +120,14 @@ typedef struct yy_engine yy_engine;
                                       simulation instead of ONE persistent kernel per search.  The persistent
                                       kernel (csrc/yy_fused.cu) is the default for the STUB and NN evaluators with
                                       leaves_per_step == 1; both produce identical trees. */
+#define YY_MODE_EVAL_RANDOM_FORM 4u /* NN evaluator: evaluate every leaf in one dihedral form of the board (the order of
+                                      augment_sample: identity, rot90 x1/x2/x3, flip left-right, flip up-down, transpose,
+                                      anti-transpose; rectangular boards: forms 0, 2, 4, 5), chosen by a hash of the position
+                                      and the engine seed: forms[mix64(stub_key(board) ^ seed) % F].  Same FLOPs as identity. */
+#define YY_MODE_EVAL_AVERAGE_FORMS 8u /* NN evaluator: evaluate every leaf in all F forms (F = 8 square, 4 rectangular) and
+                                      use the mean prior and value (fp32, ascending form order).  F x the network FLOPs and
+                                      head-feature scratch.  Excludes YY_MODE_EVAL_RANDOM_FORM.  Both modes apply to searches,
+                                      self-play and yy_evaluate; the STUB and EXTERNAL evaluators refuse them. */
 
 typedef struct {
   int32_t rows, cols;
@@ -212,6 +220,13 @@ const uint8_t *yy_engine_leaf_active(yy_engine *e);
  * out_logits float32[count][A]. */
 int yy_evaluate(yy_engine *e, const uint64_t *black_dev, const uint64_t *white_dev, int64_t count,
                 float *out_policy_dev, float *out_value_dev, float *out_logits_dev, void *stream);
+/* yy_evaluate in a given dihedral form (NN evaluator only), whatever the engine's mode_flags.  form 0..7: the network
+ * sees form `form` of every board (the form must keep the board's shape: rectangular boards take 0, 2, 4, 5) and its
+ * outputs are mapped back, so out_policy / out_logits are indexed by the board's own actions.  form -1: the mean over
+ * all forms of policy and value (no logits; needs a head-feature scratch of >= F boards: n_games x leaves_per_step >= F
+ * or YY_MODE_EVAL_AVERAGE_FORMS). */
+int yy_evaluate_form(yy_engine *e, const uint64_t *black_dev, const uint64_t *white_dev, int64_t count, int32_t form,
+                     float *out_policy_dev, float *out_value_dev, float *out_logits_dev, void *stream);
 
 /* Optional CUDA-event timing of the dominant kernel (the persistent search / forward kernel, csrc/yy_fused.cu),
  * recorded on the launching stream around every launch while enabled.  yy_engine_get_profile synchronises on the

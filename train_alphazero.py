@@ -50,6 +50,9 @@ def parse_args(argv=None):
                         "array of this package's YinYangLogic; 'reference': boards pickled as "
                         "src.yin_yang.yin_yang_logic.YinYangLogic so that the reference's own trainer loads the .npz "
                         "without this package")
+    p.add_argument("--eval-symmetry", choices=["none", "random", "average"], default="none",
+                   help="network evaluation of the search leaves in every mode: as they are (default), in one dihedral form "
+                        "of the board hashed from the position and the seed, or averaged over all forms (8x the network FLOPs)")
     return p.parse_args(argv)
 
 
@@ -77,7 +80,7 @@ def main(argv=None):
         az = AlphaZero(game=game, model_dir=args.model_dir, data_dir=args.data_dir, num_iterations=args.iterations,
                        num_episodes=args.episodes, num_simulations=args.simulations, num_epochs=args.epochs,
                        num_workers=args.workers, mcts_threads=args.mcts_threads, eval_games=args.arena_games,
-                       batch_size=args.batch_size, lr=args.lr)
+                       batch_size=args.batch_size, lr=args.lr, eval_symmetry=args.eval_symmetry)
         if args.file_loop:
             az.run()                                                     # the reference's loop: data files between the stages
         else:
@@ -102,16 +105,18 @@ def main(argv=None):
             from yinyang_game_alphazero_b200.self_play import generate_self_play_data_distributed
             data_file = generate_self_play_data_distributed(game=game, model_path=model_path, output_dir=args.data_dir,
                                                             num_games=args.episodes, num_simulations=args.simulations,
-                                                            wire=args.replay_wire)
+                                                            wire=args.replay_wire, eval_symmetry=args.eval_symmetry)
         else:
             data_file = generate_self_play_data(game=game, model_path=model_path, output_dir=args.data_dir,
                                                 num_games=args.episodes, num_workers=args.workers,
-                                                num_simulations=args.simulations, wire=args.replay_wire)
+                                                num_simulations=args.simulations, wire=args.replay_wire,
+                                                eval_symmetry=args.eval_symmetry)
         if data_file:
             logger.info(f"Self-play data generation completed. Data saved to {data_file}")
         return 0
     # evaluate: AlphaZero vs random, colours alternate (train_alphazero.py:165-243)
-    az = AlphaZeroPlayer(game=game, model_path=model_path, num_simulations=args.simulations, num_threads=args.mcts_threads)
+    az = AlphaZeroPlayer(game=game, model_path=model_path, num_simulations=args.simulations, num_threads=args.mcts_threads,
+                         eval_symmetry=args.eval_symmetry)
     rnd = RandomPlayer(game, verbose=False)
     az_wins = rnd_wins = draws = 0
     for i in range(args.eval_games):

@@ -155,6 +155,7 @@ SIGNATURES = {
     "yy_engine_leaf_white": (_P, [_P]),
     "yy_engine_leaf_active": (_P, [_P]),
     "yy_evaluate": (_I, [_P, _P, _P, _I64, _P, _P, _P, _P]),
+    "yy_evaluate_form": (_I, [_P, _P, _P, _I64, ctypes.c_int32, _P, _P, _P, _P]),
     "yy_engine_set_profiling": (_I, [_P, _I]),
     "yy_engine_get_profile": (_I, [_P, ctypes.POINTER(_I64), ctypes.POINTER(ctypes.c_double), ctypes.POINTER(_I64)]),
     "yy_engine_set_debug_stamps": (_I, [_P, _P]),

@@ -18,7 +18,7 @@ logger = logging.getLogger("YinYangGUI")
 _state = {"game": None, "player": None, "model_path": None}      # server.py:17-19 module globals
 
 
-def get_ai_move(data, num_simulations=100, num_threads=1):
+def get_ai_move(data, num_simulations=100, num_threads=1, eval_symmetry="none"):
     try:
         board_state, player = data.get("board"), data.get("currentPlayer")
         rows, cols = data.get("rows"), data.get("cols")
@@ -27,9 +27,11 @@ def get_ai_move(data, num_simulations=100, num_threads=1):
         if game is None or game.getBoardSize() != (rows, cols):
             game = _state["game"] = YinYangGame(rows, cols)
         az = _state["player"]
-        if az is None or az.game.getBoardSize() != (rows, cols) or _state["model_path"] != model_path or az.mcts.num_threads != max(1, num_threads):
+        if az is None or az.game.getBoardSize() != (rows, cols) or _state["model_path"] != model_path or az.mcts.num_threads != max(1, num_threads) \
+                or az.mcts.eval_symmetry != eval_symmetry:
             try:
-                az = _state["player"] = AlphaZeroPlayer(game=game, model_path=model_path, num_simulations=num_simulations, num_threads=num_threads)
+                az = _state["player"] = AlphaZeroPlayer(game=game, model_path=model_path, num_simulations=num_simulations, num_threads=num_threads,
+                                                      eval_symmetry=eval_symmetry)
                 _state["model_path"] = model_path
             except Exception as e:  # server.py:58-60
                 logger.error(f"Error initializing AlphaZero player: {e}", exc_info=True)

@@ -67,7 +67,7 @@ def play_match(game, current_mcts: MCTS, best_mcts: MCTS, num_games=40):
             "results": results, "plies": plies}
 
 
-def evaluate(game, current_model_path, best_model_path, num_games=40, num_simulations=800, mcts_threads=1):
+def evaluate(game, current_model_path, best_model_path, num_games=40, num_simulations=800, mcts_threads=1, eval_symmetry="none"):
     """AlphaZero.evaluate(current_model_path, best_model_path, num_games) -> win ratio of the current model."""
     logger.info(f"Evaluating {current_model_path} against {best_model_path}")
     nets = []
@@ -75,8 +75,8 @@ def evaluate(game, current_model_path, best_model_path, num_games=40, num_simula
         net = YinYangNeuralNetwork(game)
         net.load_model(path)
         nets.append(net)
-    cur = MCTS(game=game, neural_net=nets[0], num_simulations=num_simulations, num_threads=mcts_threads)
-    best = MCTS(game=game, neural_net=nets[1], num_simulations=num_simulations, num_threads=mcts_threads)
+    cur = MCTS(game=game, neural_net=nets[0], num_simulations=num_simulations, num_threads=mcts_threads, eval_symmetry=eval_symmetry)
+    best = MCTS(game=game, neural_net=nets[1], num_simulations=num_simulations, num_threads=mcts_threads, eval_symmetry=eval_symmetry)
     try:
         out = play_match(game, cur, best, num_games)
     finally:

@@ -72,22 +72,10 @@ augment_kernel(Geo<NW> g, int W, const uint64_t* __restrict__ black, const uint6
   __syncwarp();
   float* planes0 = out_planes + r * (5ll * FORMS) * A;   // [FORMS][5 planes][A]
   float* pol0 = out_policy + r * (long long)FORMS * A;   // [FORMS][A]
-  for (int a = lane; a < A; a += 32) {          // phase 2: output cell (i, j) of form f <- source cell (sx, sy)
-    const int i = a / m, j = a - i * m;         // (square boards: n == m)
+  for (int a = lane; a < A; a += 32) {          // phase 2: output cell a of form f <- source cell form_src(f, a)
 #pragma unroll
-    for (int f = 0; f < FORMS; ++f) {
-      int sx, sy;
-      switch (f) {
-        case 0: sx = i; sy = j; break;
-        case 1: sx = j; sy = m - 1 - i; break;             // np.rot90(S, 1)[i][j] = S[j][m-1-i]
-        case 2: sx = n - 1 - i; sy = m - 1 - j; break;     // rot90 x2
-        case 3: sx = n - 1 - j; sy = i; break;             // rot90 x3
-        case 4: sx = i; sy = m - 1 - j; break;             // flip left-right
-        case 5: sx = n - 1 - i; sy = j; break;             // flip up-down
-        case 6: sx = j; sy = i; break;                     // transpose
-        default: sx = n - 1 - j; sy = m - 1 - i; break;    // flip(transpose, both axes)
-      }
-      const float* sp = src + (sx * m + sy);
+    for (int f = 0; f < FORMS; ++f) {           // (square boards: n == m)
+      const float* sp = src + form_src(f, n, m, a);
       float* planes = planes0 + f * 5 * A + a;
 #pragma unroll
       for (int k = 0; k < 5; ++k) __stcs(planes + k * A, sp[k * A]);

@@ -47,6 +47,10 @@ struct FusedArgs {
                                // drops from 513 k to 93 k cycles per step) but every half streams the layer's weights again, and
                                // the weight stream (~10 B/clk per SM through the 3-slot ring) then stalls the issuer for 735 k
                                // cycles per step: 1,286 against 1,298 TFLOP/s (profiles/r02_ab_pingpong_*.txt)
+  // symmetric evaluation (FormSpec, yy_nn.cuh): the form a board is evaluated in.  Averaging walks n_avg entries per
+  // board, one per form (entry i -> board i / n_avg, form i % n_avg); the heads pass averages them in ascending form order.
+  int form_mode, form_fixed, n_avg;
+  uint64_t form_seed;
   long long* dbg;
 };
 
@@ -124,14 +128,15 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
   const int st_len = (int)clampl(a.count - (long long)(blockIdx.x - rank) * a.boards_per_cta, a.boards_per_cta);
   const bool dyn = a.mode != YY_FUSED_FORWARD;
   volatile int* cnt_s = reinterpret_cast<volatile int*>(smem + SM_CNT);   // [step parity][cluster rank][leaves, selecting]
-  int n_mine = my_len, n_struct = st_len;        // my real entries / structural length of this step's walk
+  const int E = a.n_avg;                         // walk entries per board (1 unless forms are averaged)
+  int n_mine = my_len * E, n_struct = st_len * E;   // my real entries / structural length of this step's walk
   int n_sel = 0;                                 // my games whose search continues without a leaf in this step
   bool any_work = true;
   // every thread of the CTA (pair): wait for the counts of step `iter` (written by the compaction of the step before)
   auto fetch_counts = [&](int iter) {
     if (CG == 2) cluster_sync_all(); else asm volatile("bar.sync 0;" ::: "memory");
     volatile int* c = cnt_s + (iter & 1) * 4;
-    const int c0 = c[0], c1 = CG == 2 ? c[2] : 0, s0 = c[1], s1 = CG == 2 ? c[3] : 0;
+    const int c0 = c[0] * E, c1 = CG == 2 ? c[2] * E : 0, s0 = c[1], s1 = CG == 2 ? c[3] : 0;
     n_mine = rank ? c1 : c0; n_struct = c0 > c1 ? c0 : c1; n_sel = rank ? s1 : s0;
     any_work = (c0 | c1 | s0 | s1) != 0;
   };
@@ -526,7 +531,17 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
     auto arrive_act = [&](int h = 0) { if (CG == 2) mbar_arrive_cluster(act_ready_leader[h]); else mbar_arrive(act_ready(h)); };
     // entry i of this step's walk -> board (search / self-play: the i-th game of my run that has a pending leaf)
     int32_t* my_list = dyn ? e.act_list + run_lo : nullptr;
-    auto board_of = [&](int i) -> long long { return dyn ? (long long)my_list[i] : run_lo + i; };
+    auto board_of = [&](int i) -> long long { i /= E; return dyn ? (long long)my_list[i] : run_lo + i; };
+    // the form entry i (of board `board`) is evaluated in; 0 = identity
+    auto form_of = [&](int i, long long board) -> int {
+      if (a.form_mode == YY_FORM_FIXED) return a.form_fixed;
+      if (a.form_mode == YY_FORM_AVERAGE) return form_at(i % E, g.n, g.m);
+      if (a.form_mode == YY_FORM_HASHED) {
+        const BB<NW> bb = load_bb<NW>(a.black, board, g.W) & geo.full, wb = load_bb<NW>(a.white, board, g.W) & geo.full;
+        return hashed_form(stub_key(geo, bb, wb), a.form_seed, g.n, g.m);
+      }
+      return 0;
+    };
     // One warp compacts the games of my run that have a pending leaf (from the front of my_list) and those still
     // selecting (from its back), and publishes both counts for step `iter_next` to every thread of the CTA (pair) --
     // read after the barrier in fetch_counts.
@@ -601,7 +616,9 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
                 const long long board = board_of(entry);
                 const int cell = info & 255, y = cell / g.m, x = cell % g.m;
                 const uint64_t* bb = a.black + board * g.W; const uint64_t* wb = a.white + board * g.W;
-                auto bit = [&](const uint64_t* v, int c) { return (int)((v[c >> 6] >> (c & 63)) & 1ull); };
+                // the network sees form f of the board: cell c reads cell form_src(f, c); fills are the transformed board's
+                const int f = form_of(entry, board);
+                auto bit = [&](const uint64_t* v, int c) { if (f) c = form_src(f, g.n, g.m, c); return (int)((v[c >> 6] >> (c & 63)) & 1ull); };
                 const int isb = bit(bb, cell), isw = bit(wb, cell);
                 int rc = 0, cc = 0;
                 for (int xx = 0; xx < g.m; ++xx) { int c = y * g.m + xx; rc += bit(bb, c) | bit(wb, c); }
@@ -674,7 +691,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
                 }
                 if (is_conv1) tc_wait_st();
               } else {
-                __nv_bfloat16* dst = a.headfeat + (size_t)(run_lo + entry) * (TW_HEADC * g.A) + (info & 255);   // by walk entry
+                __nv_bfloat16* dst = a.headfeat + (size_t)(run_lo * E + entry) * (TW_HEADC * g.A) + (info & 255);   // by walk entry
                 const int h_n = n_c >= 2 ? n_c / 2 : 1, h_lo = n_c >= 2 ? c_lo / 2 : c_lo;   // 4 chunks of 16 head channels over the same warps
 #pragma unroll 1
                 for (int cc = h_lo; cc < h_lo + h_n && cc < TW_HEADC / 16; ++cc) {
@@ -758,7 +775,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
             if (q > 0) { wait_acc(); sub(6); }   // previous panel consumed
             const int nchunks = panel_stages(p) * 8;
             const int kbase = p * FC_PANEL_STAGES * 64;
-            const __nv_bfloat16* src0 = a.headfeat + (size_t)(run_lo + bb0) * (TW_HEADC * g.A) + (size_t)h * fc.Kh + kbase;
+            const __nv_bfloat16* src0 = a.headfeat + (size_t)(run_lo * E + bb0) * (TW_HEADC * g.A) + (size_t)h * fc.Kh + kbase;
             for (int idx = etid; idx < nbb * nchunks; idx += TW_EPI_THREADS) {
               const int b = idx / nchunks, j = idx - b * nchunks;
               const bool valid = kbase + j * 8 < fc.Kh;      // K padding up to the stage boundary must be zero
@@ -806,24 +823,43 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
 
         // ---- per board: softmax over all A logits (predict, neural_network.py:152), value_fc2 + tanh (:121), tree step
         if (dyn && slim == n_struct && etid == 0) *(cnt_s + 8) = iter + 1;    // last tree phase of the step: background warps wind up
-        for (int b = ew; b < nbb; b += TW_EPI_WARPS) {
-          const long long board = board_of(bb0 + b);
+        // (one warp per board: its E entries are consecutive and in this batch, since E divides batch_boards)
+        for (int b0e = ew * E; b0e < nbb; b0e += TW_EPI_WARPS * E) {
+          const long long board = board_of(bb0 + b0e);
           if (a.use_nn) {
-            const float* lg = sc_logit + b * 256;
-            float mx = -INFINITY;
-            for (int k = lane; k < g.A; k += 32) mx = fmaxf(mx, lg[k]);
-            for (int off = 16; off; off >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
-            float sum = 0.0f;
-            for (int k = lane; k < g.A; k += 32) sum += expf(lg[k] - mx);
-            for (int off = 16; off; off >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, off);
-            for (int k = lane; k < g.A; k += 32) {
-              a.policy[board * g.A + k] = expf(lg[k] - mx) / sum;
-              if (a.logits) a.logits[board * g.A + k] = lg[k];
+            float vsum = 0.0f;
+            for (int q = 0; q < E; ++q) {
+              const int b = b0e + q;
+              const int f = form_of(bb0 + b, board);
+              const float* lg = sc_logit + b * 256;
+              float mx = -INFINITY;
+              for (int k = lane; k < g.A; k += 32) mx = fmaxf(mx, lg[k]);
+              for (int off = 16; off; off >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
+              float sum = 0.0f;
+              for (int k = lane; k < g.A; k += 32) sum += expf(lg[k] - mx);
+              for (int off = 16; off; off >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, off);
+              // output k of form f is the prior (logit) of action form_src(f, k); averaging: fp32 sum in ascending form
+              // order, then / E (a power of two: exact)
+              for (int k = lane; k < g.A; k += 32) {
+                const long long o = board * g.A + (f ? form_src(f, g.n, g.m, k) : k);
+                const float p = expf(lg[k] - mx) / sum;
+                if (E == 1) {
+                  a.policy[o] = p;
+                  if (a.logits) a.logits[o] = lg[k];
+                } else {
+                  const float s = q ? a.policy[o] + p : p;
+                  a.policy[o] = q + 1 == E ? s * (1.0f / (float)E) : s;
+                }
+              }
+              float acc = 0.0f;
+              for (int k = lane; k < 256; k += 32) acc += sc_hidden[b * 256 + k];
+              for (int off = 16; off; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+              const float v = tanhf(acc + __ldg(a.fc_value2_b));
+              if (E == 1) { if (lane == 0) a.value[board] = v; }
+              else vsum += v;
+              __syncwarp();
             }
-            float acc = 0.0f;
-            for (int k = lane; k < 256; k += 32) acc += sc_hidden[b * 256 + k];
-            for (int off = 16; off; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
-            if (lane == 0) a.value[board] = tanhf(acc + __ldg(a.fc_value2_b));
+            if (E > 1 && lane == 0) a.value[board] = vsum * (1.0f / (float)E);
             __syncwarp();
           }
           if (dyn) {
@@ -881,13 +917,21 @@ static int launch_fused(NNState& nn, const FusedArgs& fa, const EngineDev& dev, 
 //   dev == nullptr : plain forward (do_tree off); policy/value/logits are the caller's output arrays.
 //   dev != nullptr : whole search over dev->leaf_* / eval_* (slot = game; leaves_per_step must be 1).
 int nn_fused_run(NNState& nn, const EngineDev* dev, uint32_t rule_flags, const uint64_t* black, const uint64_t* white, int64_t count,
-                 float* policy, float* value, float* logits, int iterations, bool use_nn, int mode, cudaStream_t s) {
+                 float* policy, float* value, float* logits, int iterations, bool use_nn, int mode, const FormSpec& forms,
+                 cudaStream_t s) {
   if (use_nn) {
     if (!nn.attrs_set) return set_error(YY_ERR_STATE, "engine was not created with the NN evaluator");
     if (!nn.weights) return set_error(YY_ERR_STATE, "no weights loaded (yy_engine_load_weights)");
   }
+  if (forms.mode != YY_FORM_IDENTITY && !use_nn) return set_error(YY_ERR_INVALID, "symmetric evaluation needs the NN evaluator");
+  if (forms.mode == YY_FORM_FIXED && !form_valid(forms.form, nn.rows, nn.cols))
+    return set_error(YY_ERR_INVALID, "form %d is not a form of a %dx%d board", forms.form, nn.rows, nn.cols);
+  if (forms.mode == YY_FORM_AVERAGE && logits) return set_error(YY_ERR_INVALID, "no logits when averaging over the forms");
+  const int E = form_entries(forms.mode, nn.rows, nn.cols);
   if (count <= 0 || iterations <= 0) return YY_OK;
-  if (count > nn.max_boards) return set_error(YY_ERR_INVALID, "fused run: %lld boards exceed the head-feature scratch (%d)", (long long)count, nn.max_boards);
+  if (count > nn.max_boards || count * E > nn.max_entries)
+    return set_error(YY_ERR_INVALID, "fused run: %lld boards x %d forms exceed the head-feature scratch (%d boards, %d entries)",
+                     (long long)count, E, nn.max_boards, nn.max_entries);
   if ((mode != YY_FUSED_FORWARD) != (dev != nullptr)) return set_error(YY_ERR_INVALID, "fused run: mode / engine state mismatch");
   FusedArgs fa{};
   fa.g = make_fused_geo(nn.rows, nn.cols, nn.blocks);
@@ -911,6 +955,8 @@ int nn_fused_run(NNState& nn, const EngineDev* dev, uint32_t rule_flags, const u
   fa.split_halves = nn.dbg_flags & 1;
   fa.no_skew = (nn.dbg_flags >> 1) & 1;
   fa.batch_boards = fused_batch_boards(fa.g);
+  fa.form_mode = forms.mode; fa.form_fixed = forms.form; fa.form_seed = forms.seed; fa.n_avg = E;
+  fa.batch_boards -= fa.batch_boards % E;   // a board's E entries share a heads pass (E in {1, 4, 8} <= every batch)
   // equal contiguous runs of boards per CTA (a search keeps its games on the same SM from the first to the last simulation)
   int sms = nn.num_sms > 0 ? nn.num_sms : 148;
   // (small batches -- an arena of 16 games, a search of a few hundred positions -- are spread over as many CTAs as there are boards

@@ -20,11 +20,16 @@ int64_t nn_weight_bytes(int rows, int cols, int channels, int blocks) {
   return weight_layout(rows, cols, blocks).total;
 }
 
-// engine scratch = the head-conv features [max_boards][64*A] bf16 (written and re-read by the same CTA: an L2 round trip)
+// walk entries per board of the head-feature scratch: one per form when the engine averages over the forms
+static int scratch_entries_per_board(const yy_engine_config& cfg) {
+  return (cfg.mode_flags & YY_MODE_EVAL_AVERAGE_FORMS) ? form_count(cfg.rows, cfg.cols) : 1;
+}
+
+// engine scratch = the head-conv features [max_entries][64*A] bf16 (written and re-read by the same CTA: an L2 round trip)
 size_t nn_workspace_bytes(const yy_engine_config& cfg) {
   if (cfg.evaluator != YY_EVAL_NN) return 0;
   const int64_t boards = (int64_t)cfg.n_games * (cfg.leaves_per_step > 0 ? cfg.leaves_per_step : 1);
-  return (size_t)align256(boards * TW_HEADC * cfg.rows * cfg.cols * 2);
+  return (size_t)align256(boards * scratch_entries_per_board(cfg) * TW_HEADC * cfg.rows * cfg.cols * 2);
 }
 
 int nn_init(NNState& nn, const yy_engine_config& cfg, void* scratch) {
@@ -32,6 +37,7 @@ int nn_init(NNState& nn, const yy_engine_config& cfg, void* scratch) {
   nn.rows = cfg.rows; nn.cols = cfg.cols; nn.A = cfg.rows * cfg.cols; nn.W = words_for_cells(nn.A);
   nn.channels = cfg.nn_channels; nn.blocks = cfg.nn_blocks;
   nn.max_boards = cfg.n_games * (cfg.leaves_per_step > 0 ? cfg.leaves_per_step : 1); nn.device = cfg.device;
+  nn.max_entries = nn.max_boards * scratch_entries_per_board(cfg);
   if (cfg.evaluator != YY_EVAL_NN) return YY_OK;
   if (!nn_geometry_ok(cfg.rows, cfg.cols) || cfg.nn_channels > TW_C)
     return set_error(YY_ERR_INVALID, "network geometry unsupported: %dx%d, %d channels", cfg.rows, cfg.cols, cfg.nn_channels);

@@ -7,7 +7,8 @@ namespace yy {
 
 struct NNState {
   int rows, cols, A, W, channels, blocks;
-  int max_boards;            // capacity of the head-feature scratch (>= n_games)
+  int max_boards;            // boards per launch (>= n_games)
+  int max_entries;           // capacity of the head-feature scratch in walk entries (max_boards x forms when averaging)
   const void* weights;       // packed image (device), owned by the caller
   int64_t weight_bytes;
   void* scratch;             // head features etc. (inside the engine workspace)
@@ -40,7 +41,19 @@ struct EngineDev;
 //                     the same step (sp_advance_game), within its move budget and the game quota.
 // use_nn = false runs the deterministic-prior evaluator (tree steps only).
 enum { YY_FUSED_FORWARD = 0, YY_FUSED_SEARCH = 1, YY_FUSED_SELFPLAY = 2 };
+// Symmetric evaluation: the dihedral form (form_src, yy_rules.cuh) the network sees a board in.
+//   IDENTITY  the board as it is;  FIXED  form `form` for every board;  HASHED  form hashed_form(stub_key(board), seed);
+//   AVERAGE   every valid form, policy and value averaged over them (fp32, ascending form order; no logits).
+enum { YY_FORM_IDENTITY = 0, YY_FORM_FIXED = 1, YY_FORM_HASHED = 2, YY_FORM_AVERAGE = 3 };
+struct FormSpec {
+  int mode = YY_FORM_IDENTITY;
+  int form = 0;
+  uint64_t seed = 0;
+};
+// walk entries (head-feature rows) per board under a form mode
+inline int form_entries(int mode, int rows, int cols) { return mode == YY_FORM_AVERAGE ? form_count(rows, cols) : 1; }
 int nn_fused_run(NNState& nn, const EngineDev* dev, uint32_t rule_flags, const uint64_t* black, const uint64_t* white,
-                 int64_t count, float* policy, float* value, float* logits, int iterations, bool use_nn, int mode, cudaStream_t stream);
+                 int64_t count, float* policy, float* value, float* logits, int iterations, bool use_nn, int mode,
+                 const FormSpec& forms, cudaStream_t stream);
 
 }  // namespace yy

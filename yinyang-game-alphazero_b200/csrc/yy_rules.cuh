@@ -272,4 +272,34 @@ YY_HD float stub_value(uint64_t key) {
   return (float)((int32_t)(mix64(key ^ 0xA0761D6478BD642Full) >> 47) - 65536) * (1.0f / 65536.0f);
 }
 
+// ---- the dihedral forms of a board, in augment_sample's order (data_utils.py:59-76): 0 identity, 1-3 rot90 x1/x2/x3
+// counter-clockwise, 4 flip left-right, 5 flip up-down, 6 transpose, 7 anti-transpose.  Form f of a board S shows at
+// cell c the cell form_src(f, c) of S.  The training data (yy_dataset.cu) and the network's symmetric evaluation
+// (yy_fused.cu: the stem reads S[form_src(f, c)], output c is the prior of action form_src(f, c)) share this map.
+// A rectangular board keeps its shape only under forms 0, 2, 4, 5.
+YY_HD int form_count(int rows, int cols) { return rows == cols ? 8 : 4; }
+YY_HD int form_at(int k, int rows, int cols) { return rows == cols ? k : (k < 2 ? 2 * k : k + 2); }   // k-th valid form
+YY_HD bool form_valid(int f, int rows, int cols) {
+  return f >= 0 && f < 8 && (rows == cols || f == 0 || f == 2 || f == 4 || f == 5);
+}
+YY_HD int form_src(int f, int n, int m, int c) {
+  const int i = c / m, j = c - i * m;
+  int sx, sy;
+  switch (f) {
+    case 0: sx = i; sy = j; break;
+    case 1: sx = j; sy = m - 1 - i; break;             // np.rot90(S, 1)[i][j] = S[j][m-1-i]
+    case 2: sx = n - 1 - i; sy = m - 1 - j; break;     // rot90 x2
+    case 3: sx = n - 1 - j; sy = i; break;             // rot90 x3
+    case 4: sx = i; sy = m - 1 - j; break;             // flip left-right
+    case 5: sx = n - 1 - i; sy = j; break;             // flip up-down
+    case 6: sx = j; sy = i; break;                     // transpose
+    default: sx = n - 1 - j; sy = m - 1 - i; break;    // flip(transpose, both axes)
+  }
+  return sx * m + sy;
+}
+// form of a position under random-form evaluation: a pure function of (engine seed, position)
+YY_HD int hashed_form(uint64_t key, uint64_t seed, int rows, int cols) {
+  return form_at((int)(mix64(key ^ seed) % (uint64_t)form_count(rows, cols)), rows, cols);
+}
+
 }  // namespace yy

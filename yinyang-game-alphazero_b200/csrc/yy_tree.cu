@@ -130,6 +130,10 @@ static int normalise_cfg(yy_engine_config& c) {
   if (c.nn_blocks < 0) c.nn_blocks = 10;
   if (c.leaves_per_step < 1) c.leaves_per_step = 1;
   if (c.leaves_per_step > 64) return set_error(YY_ERR_INVALID, "leaves_per_step must be <= 64");
+  const uint32_t sym = c.mode_flags & (YY_MODE_EVAL_RANDOM_FORM | YY_MODE_EVAL_AVERAGE_FORMS);
+  if (sym == (YY_MODE_EVAL_RANDOM_FORM | YY_MODE_EVAL_AVERAGE_FORMS))
+    return set_error(YY_ERR_INVALID, "YY_MODE_EVAL_RANDOM_FORM and YY_MODE_EVAL_AVERAGE_FORMS exclude each other");
+  if (sym && c.evaluator != YY_EVAL_NN) return set_error(YY_ERR_INVALID, "symmetric evaluation needs the NN evaluator");
   // in-flight simulations each own a node: keep the worst case inside the node arena
   return YY_OK;
 }
@@ -200,13 +204,25 @@ int launch_step(yy_engine* e, cudaStream_t s) {
   YY_LAUNCH_CHECK();
   return YY_OK;
 }
-// network forward = the persistent kernel with one iteration and no tree step
+// the form every network evaluation of the engine uses (mode_flags)
+FormSpec engine_forms(const yy_engine* e) {
+  FormSpec f;
+  if (e->cfg.mode_flags & YY_MODE_EVAL_RANDOM_FORM) { f.mode = YY_FORM_HASHED; f.seed = e->cfg.seed; }
+  if (e->cfg.mode_flags & YY_MODE_EVAL_AVERAGE_FORMS) f.mode = YY_FORM_AVERAGE;
+  return f;
+}
+// network forward = the persistent kernel with one iteration and no tree step (in chunks that fit the head-feature scratch)
 int engine_forward(yy_engine* e, const uint64_t* black, const uint64_t* white, int64_t count, float* policy, float* value,
-                   float* logits, cudaStream_t s) {
-  for (int64_t done = 0; done < count; done += e->nn.max_boards) {
-    const int64_t n = (count - done) < e->nn.max_boards ? (count - done) : e->nn.max_boards;
+                   float* logits, const FormSpec& forms, cudaStream_t s) {
+  const int E = form_entries(forms.mode, e->cfg.rows, e->cfg.cols);
+  int64_t chunk = e->nn.max_entries / E < e->nn.max_boards ? e->nn.max_entries / E : e->nn.max_boards;
+  if (chunk < 1)
+    return set_error(YY_ERR_INVALID, "averaging over %d forms needs a head-feature scratch of >= %d boards (n_games x leaves_per_step), "
+                     "or an engine created with YY_MODE_EVAL_AVERAGE_FORMS", E, E);
+  for (int64_t done = 0; done < count; done += chunk) {
+    const int64_t n = (count - done) < chunk ? (count - done) : chunk;
     int rc = nn_fused_run(e->nn, nullptr, e->cfg.rule_flags, black + done * e->dev.W, white + done * e->dev.W, n, policy + done * e->dev.A,
-                          value + done, logits ? logits + done * e->dev.A : nullptr, 1, true, YY_FUSED_FORWARD, s);
+                          value + done, logits ? logits + done * e->dev.A : nullptr, 1, true, YY_FUSED_FORWARD, forms, s);
     if (rc) return rc;
   }
   return YY_OK;
@@ -215,7 +231,8 @@ int engine_forward(yy_engine* e, const uint64_t* black, const uint64_t* white, i
 int run_evaluator(yy_engine* e, cudaStream_t s) {
   if (e->cfg.evaluator == YY_EVAL_STUB) return YY_OK;
   if (e->cfg.evaluator == YY_EVAL_NN)
-    return engine_forward(e, e->dev.leaf_black, e->dev.leaf_white, e->dev.n_slots, e->dev.eval_prior, e->dev.eval_value, nullptr, s);
+    return engine_forward(e, e->dev.leaf_black, e->dev.leaf_white, e->dev.n_slots, e->dev.eval_prior, e->dev.eval_value, nullptr,
+                          engine_forms(e), s);
   return set_error(YY_ERR_STATE, "external evaluator: use yy_search_begin / yy_search_advance");
 }
 // full search over the roots already stored in dev.root_* (noise pointers already set in dev)
@@ -225,7 +242,8 @@ int search_core(yy_engine* e, cudaStream_t s) {
     // the whole search in ONE persistent kernel: every CTA owns a run of games from the first to the last simulation
     // (the launch ends as soon as no game has work left; a game advances by at least one simulation every two steps)
     return nn_fused_run(e->nn, &e->dev, e->cfg.rule_flags, e->dev.leaf_black, e->dev.leaf_white, e->dev.n_slots, e->dev.eval_prior,
-                        e->dev.eval_value, nullptr, 2 * (e->cfg.n_sims + 1), e->cfg.evaluator == YY_EVAL_NN, YY_FUSED_SEARCH, s);
+                        e->dev.eval_value, nullptr, 2 * (e->cfg.n_sims + 1), e->cfg.evaluator == YY_EVAL_NN, YY_FUSED_SEARCH,
+                        engine_forms(e), s);
   }
   if (e->cfg.leaves_per_step <= 1) {      // deterministic mode: exactly n_sims + 1 lock-steps, no host synchronisation
     for (int i = 0; i <= e->cfg.n_sims; ++i) {
@@ -386,7 +404,7 @@ int yy_evaluate(yy_engine* e, const uint64_t* black, const uint64_t* white, int6
   if (!e || !black || !white || !out_policy || !out_value) return set_error(YY_ERR_INVALID, "null argument");
   if (count <= 0) return YY_OK;
   cudaStream_t s = (cudaStream_t)stream;
-  if (e->cfg.evaluator == YY_EVAL_NN) return engine_forward(e, black, white, count, out_policy, out_value, out_logits, s);
+  if (e->cfg.evaluator == YY_EVAL_NN) return engine_forward(e, black, white, count, out_policy, out_value, out_logits, engine_forms(e), s);
   if (e->cfg.evaluator == YY_EVAL_STUB) {
     YY_DISPATCH_NW(e->dev.A, stub_eval_kernel<NW><<<thread_grid((int)count, 128), 128, 0, s>>>(
         make_geo<NW>(e->cfg.rows, e->cfg.cols, e->cfg.rule_flags), e->dev.W, black, white, count, out_policy, out_value));
@@ -394,6 +412,20 @@ int yy_evaluate(yy_engine* e, const uint64_t* black, const uint64_t* white, int6
     return YY_OK;
   }
   return set_error(YY_ERR_STATE, "yy_evaluate needs the STUB or NN evaluator");
+}
+
+int yy_evaluate_form(yy_engine* e, const uint64_t* black, const uint64_t* white, int64_t count, int32_t form, float* out_policy,
+                     float* out_value, float* out_logits, void* stream) {
+  if (!e || !black || !white || !out_policy || !out_value) return set_error(YY_ERR_INVALID, "null argument");
+  if (e->cfg.evaluator != YY_EVAL_NN) return set_error(YY_ERR_INVALID, "yy_evaluate_form needs the NN evaluator");
+  FormSpec f;
+  if (form == -1) f.mode = YY_FORM_AVERAGE;
+  else if (form_valid(form, e->cfg.rows, e->cfg.cols)) { f.mode = YY_FORM_FIXED; f.form = form; }
+  else return set_error(YY_ERR_INVALID, "form %d is not a form of a %dx%d board (0..7 square, 0/2/4/5 rectangular; -1 = average)",
+                        form, e->cfg.rows, e->cfg.cols);
+  if (f.mode == YY_FORM_AVERAGE && out_logits) return set_error(YY_ERR_INVALID, "no logits when averaging over the forms");
+  if (count <= 0) return YY_OK;
+  return engine_forward(e, black, white, count, out_policy, out_value, out_logits, f, (cudaStream_t)stream);
 }
 
 int yy_engine_set_profiling(yy_engine* e, int enable) {
@@ -437,7 +469,8 @@ static int launch_rolling(yy_engine* e, int moves_per_slot, long long iterations
   YY_LAUNCH_CHECK();
   if (iterations > 0x7fffffffll) iterations = 0x7fffffffll;
   return nn_fused_run(e->nn, &e->dev, e->cfg.rule_flags, e->dev.leaf_black, e->dev.leaf_white, e->dev.n_slots, e->dev.eval_prior,
-                      e->dev.eval_value, nullptr, (int)iterations, e->cfg.evaluator == YY_EVAL_NN, YY_FUSED_SELFPLAY, s);
+                      e->dev.eval_value, nullptr, (int)iterations, e->cfg.evaluator == YY_EVAL_NN, YY_FUSED_SELFPLAY,
+                      engine_forms(e), s);
 }
 
 int yy_selfplay_run(yy_engine* e, int32_t n_moves, void* stream) {

@@ -65,13 +65,14 @@ class DeviceSelfPlay:
     """Rolling self-play whose finished games stay on the device (engine replay ring -> device tensors)."""
 
     def __init__(self, game, state_dict, slots=4096, num_simulations=800, temperature_threshold=10, dirichlet_alpha=0.3,
-                 dirichlet_epsilon=0.25, cpuct=1.0, seed=0, evaluator="nn", device=None):
+                 dirichlet_epsilon=0.25, cpuct=1.0, seed=0, evaluator="nn", device=None, eval_symmetry="none"):
         self.n, self.m = game.getBoardSize()
         self.A, self.slots, self.sims = self.n * self.m, int(slots), int(num_simulations)
         self.eng = _engine.Engine(rows=self.n, cols=self.m, n_games=self.slots, n_sims=self.sims, evaluator=evaluator, cpuct=cpuct,
                                   rule_flags=getattr(game, "rule_flags", 0), dirichlet_alpha=dirichlet_alpha,
                                   dirichlet_epsilon=dirichlet_epsilon, temperature_threshold=temperature_threshold, seed=seed,
-                                  state_dict=state_dict, replay_capacity=self.slots * (2 * self.A + 8) + 4096, device=device)
+                                  state_dict=state_dict, replay_capacity=self.slots * (2 * self.A + 8) + 4096, device=device,
+                                  eval_symmetry=eval_symmetry)
         self.cursor, self._pend = 0, None
         self.games_done = 0
 
@@ -123,8 +124,9 @@ class DeviceLoop:
     def __init__(self, game, model_dir="models", num_iterations=100, num_episodes=100, num_simulations=800, num_epochs=10,
                  batch_size=64, lr=0.001, weight_decay=1e-4, sample_size=10000, queue_size=500000, update_threshold=0.6, eval_games=40,
                  num_channels=128, num_res_blocks=10, slots=4096, temperature_threshold=10, exact_episodes=False, save_files=True,
-                 seed=0, mcts_threads=1, state_dict=None):
+                 seed=0, mcts_threads=1, state_dict=None, eval_symmetry="none"):
         self.game, self.model_dir = game, model_dir
+        self.eval_symmetry = eval_symmetry
         self.num_iterations, self.num_episodes, self.num_simulations, self.num_epochs = num_iterations, num_episodes, num_simulations, num_epochs
         self.batch_size, self.sample_size, self.update_threshold, self.eval_games = batch_size, sample_size, update_threshold, eval_games
         self.exact_episodes, self.save_files, self.mcts_threads = exact_episodes, save_files, mcts_threads
@@ -140,7 +142,8 @@ class DeviceLoop:
         share = -(-num_episodes // self.world)
         self.episodes_per_rank = share
         self.selfplay = DeviceSelfPlay(game, self.best_sd, slots=max(1, min(slots, share)), num_simulations=num_simulations,
-                                       temperature_threshold=temperature_threshold, seed=seed * 1000003 + self.rank)
+                                       temperature_threshold=temperature_threshold, seed=seed * 1000003 + self.rank,
+                                       eval_symmetry=eval_symmetry)
         self.buffer = DeviceReplayBuffer(self.selfplay.eng.W, n * m, queue_size)
         self.gen = torch.Generator(device="cuda")
         self.gen.manual_seed(seed * 7919 + self.rank)
@@ -199,8 +202,10 @@ class DeviceLoop:
                 net = YinYangNeuralNetwork(self.game, C, B)
                 net.load_state_dict(sd)
                 nets.append(net)
-            cur = MCTS(self.game, nets[0], num_simulations=self.num_simulations, num_threads=self.mcts_threads, verbose=0)
-            best = MCTS(self.game, nets[1], num_simulations=self.num_simulations, num_threads=self.mcts_threads, verbose=0)
+            cur = MCTS(self.game, nets[0], num_simulations=self.num_simulations, num_threads=self.mcts_threads, verbose=0,
+                       eval_symmetry=self.eval_symmetry)
+            best = MCTS(self.game, nets[1], num_simulations=self.num_simulations, num_threads=self.mcts_threads, verbose=0,
+                        eval_symmetry=self.eval_symmetry)
             try:
                 ratio = arena.play_match(self.game, cur, best, self.eval_games)["win_ratio"]
             finally:

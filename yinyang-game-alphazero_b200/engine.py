@@ -21,6 +21,17 @@ RULE_ROWCOL = 1
 EVAL_STUB, EVAL_NN, EVAL_EXTERNAL = 0, 1, 2
 MODE_SEARCH_AS_BLACK = 1
 MODE_STEP_KERNELS = 2
+MODE_EVAL_RANDOM_FORM = 4
+MODE_EVAL_AVERAGE_FORMS = 8
+# eval_symmetry -> mode_flags: evaluate every leaf as it is, in one form hashed from (seed, position), or averaged over all
+# dihedral forms (include/yinyang_b200.h, YY_MODE_EVAL_*)
+EVAL_SYMMETRY = {"none": 0, "random": MODE_EVAL_RANDOM_FORM, "average": MODE_EVAL_AVERAGE_FORMS}
+
+
+def symmetry_forms(rows, cols):
+    """The dihedral forms that keep a rows x cols board's shape, in augment_sample's order (0 identity, 1-3 rot90 x1/x2/x3,
+    4 flip left-right, 5 flip up-down, 6 transpose, 7 anti-transpose)."""
+    return list(range(8)) if rows == cols else [0, 2, 4, 5]
 RESULT_DRAW_CODE = 2
 DRAW_VALUE = 0.0001  # yin_yang_game.py:107
 
@@ -292,7 +303,11 @@ class Engine:
     def __init__(self, rows=8, cols=8, n_games=1, n_sims=800, evaluator="stub", cpuct=1.0, rule_flags=0,
                  search_as_black=True, edges_per_game=0, dirichlet_alpha=0.3, dirichlet_epsilon=0.25,
                  temperature_threshold=10, seed=0, replay_capacity=0, state_dict=None, nn_channels=128, nn_blocks=10,
-                 device=None, leaves_per_step=1, step_kernels=False, descents_per_step=0):
+                 device=None, leaves_per_step=1, step_kernels=False, descents_per_step=0, eval_symmetry="none"):
+        if eval_symmetry not in EVAL_SYMMETRY:
+            raise ValueError(f"eval_symmetry must be one of {sorted(EVAL_SYMMETRY)}, not {eval_symmetry!r}")
+        if eval_symmetry != "none" and evaluator != "nn":
+            raise ValueError("eval_symmetry needs evaluator='nn'")
         _require_cuda()
         self.L = _lib.lib()
         self.rows, self.cols, self.A, self.W = rows, cols, rows * cols, bitboard.words_for(rows, cols)
@@ -303,6 +318,7 @@ class Engine:
         self.tdev = torch.device("cuda", self.device)
         ev = {"stub": EVAL_STUB, "nn": EVAL_NN, "external": EVAL_EXTERNAL}[evaluator]
         self.evaluator = evaluator
+        self.eval_symmetry = eval_symmetry
         if evaluator == "nn":
             if state_dict is None:
                 raise ValueError("evaluator='nn' needs a reference state_dict / checkpoint dict")
@@ -311,7 +327,8 @@ class Engine:
         if replay_capacity <= 0:
             replay_capacity = max(1, n_games * (self.A + 8))
         self.cfg = _lib.EngineConfig(rows=rows, cols=cols, n_games=n_games, n_sims=n_sims, rule_flags=rule_flags,
-                                     mode_flags=(MODE_SEARCH_AS_BLACK if search_as_black else 0) | (MODE_STEP_KERNELS if step_kernels else 0), evaluator=ev,
+                                     mode_flags=(MODE_SEARCH_AS_BLACK if search_as_black else 0) | (MODE_STEP_KERNELS if step_kernels else 0)
+                                     | EVAL_SYMMETRY[eval_symmetry], evaluator=ev,
                                      edges_per_game=edges_per_game, temperature_threshold=temperature_threshold,
                                      replay_capacity=replay_capacity, nn_channels=nn_channels, nn_blocks=nn_blocks,
                                      device=self.device, leaves_per_step=self.leaves_per_step, cpuct=cpuct, descents_per_step=int(descents_per_step),
@@ -454,18 +471,30 @@ class Engine:
         return counts, cw
 
     # -- evaluator on an arbitrary batch (batched predict)
-    def evaluate(self, black, white, want_logits=False):
+    def evaluate(self, black, white, want_logits=False, form=None):
+        """form=None: the engine's own eval_symmetry; an int: that dihedral form (symmetry_forms), outputs mapped back to
+        the board's actions; "average": policy and value averaged over all forms (no logits)."""
         n = black.shape[0]
         policy = torch.empty((n, self.A), dtype=torch.float32, device=self.tdev)
         value = torch.empty(n, dtype=torch.float32, device=self.tdev)
         logits = torch.empty((n, self.A), dtype=torch.float32, device=self.tdev) if want_logits else None
-        _lib.check(self.L.yy_evaluate(self.handle, _ptr(black), _ptr(white), n, _ptr(policy), _ptr(value), _ptr(logits),
-                                      _stream()))
+        if form is None:
+            _lib.check(self.L.yy_evaluate(self.handle, _ptr(black), _ptr(white), n, _ptr(policy), _ptr(value), _ptr(logits),
+                                          _stream()))
+        else:
+            if form == "average":
+                code = -1
+            elif isinstance(form, (int, np.integer)) and not isinstance(form, bool) and 0 <= int(form) <= 7:
+                code = int(form)
+            else:
+                raise ValueError(f"form must be None, 0..7 or 'average', not {form!r}")
+            _lib.check(self.L.yy_evaluate_form(self.handle, _ptr(black), _ptr(white), n, code, _ptr(policy), _ptr(value),
+                                               _ptr(logits), _stream()))
         return (policy, value, logits) if want_logits else (policy, value)
 
-    def evaluate_host(self, boards, want_logits=False):
+    def evaluate_host(self, boards, want_logits=False, form=None):
         b, w = bitboard.pack_boards(boards, self.rows, self.cols)
-        out = self.evaluate(_to_dev(b, torch.int64), _to_dev(w, torch.int64), want_logits)
+        out = self.evaluate(_to_dev(b, torch.int64), _to_dev(w, torch.int64), want_logits, form=form)
         return tuple(o.cpu().numpy() for o in out)
 
     # -- profiling of the dominant kernel

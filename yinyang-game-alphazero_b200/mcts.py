@@ -107,8 +107,11 @@ ChildStats = RootView = Node      # names of the round-1 facade
 
 class MCTS:
     def __init__(self, game, neural_net, num_simulations=800, cpuct=1.0, temperature=1.0, num_threads=1,
-                 dirichlet_noise=True, dirichlet_alpha=0.3, dirichlet_epsilon=0.25, verbose=1):
+                 dirichlet_noise=True, dirichlet_alpha=0.3, dirichlet_epsilon=0.25, verbose=1, eval_symmetry="none"):
         self.game, self.neural_net = game, neural_net
+        # network evaluations of the leaves: "none" as they are, "random" in one dihedral form hashed from (seed, position),
+        # "average" averaged over all forms (Engine(eval_symmetry=); network evaluator only)
+        self.eval_symmetry = eval_symmetry
         self.num_simulations, self.cpuct, self.temperature = num_simulations, cpuct, temperature
         # mcts.py:320-321,414-426 runs the simulations of a search on `num_threads` threads; here num_threads = K > 1 selects
         # K leaves per game per step with virtual loss (Engine(leaves_per_step=K)): K simulations share one network batch,
@@ -139,6 +142,8 @@ class MCTS:
                       dirichlet_epsilon=self.dirichlet_epsilon)
             if self._mode() == "nn":
                 kw["state_dict"] = self.neural_net.state_dict()
+            if self.eval_symmetry != "none":
+                kw["eval_symmetry"] = self.eval_symmetry
             if self.num_threads > 1 and self._mode() != "external":
                 kw["leaves_per_step"] = self.num_threads
             e = self._engines[n_games] = _engine.Engine(**kw)

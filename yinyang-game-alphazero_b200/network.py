@@ -56,8 +56,9 @@ def safe_load(filename):
 class YinYangNeuralNetwork:
     """Drop-in for the evaluator role of the reference class: predict / load_model / save_model."""
 
-    def __init__(self, game, num_channels=128, num_res_blocks=10):
+    def __init__(self, game, num_channels=128, num_res_blocks=10, eval_symmetry="none"):
         self.game = game
+        self.eval_symmetry = eval_symmetry     # predict(): "none", "random" (hashed form) or "average" (Engine(eval_symmetry=))
         self.board_size = game.getBoardSize()
         self.action_size = game.getActionSize()
         self.input_channels = 5
@@ -96,7 +97,8 @@ class YinYangNeuralNetwork:
                 self._engine.close()
             n, m = self.board_size
             self._engine = _engine.Engine(rows=n, cols=m, n_games=n_games, n_sims=1, evaluator="nn",
-                                          state_dict=self.state_dict(), rule_flags=getattr(self.game, "rule_flags", 0))
+                                          state_dict=self.state_dict(), rule_flags=getattr(self.game, "rule_flags", 0),
+                                          eval_symmetry=self.eval_symmetry)
         return self._engine
 
     def predict(self, board):  # neural_network.py:125-154 -> (float32[A] softmax over ALL actions, np.float32)

@@ -34,15 +34,16 @@ class AlphaZeroPlayer:
     """MCTS-backed player (alphazero.py:272-364): search as player 1 on the canonical (= identical) board,
     temperature 0, mask with the real player's legal moves, random legal fallback."""
 
-    def __init__(self, game, model_path, num_simulations=800, num_threads=1):
+    def __init__(self, game, model_path, num_simulations=800, num_threads=1, eval_symmetry="none"):
         self.game = game
-        self.neural_net = YinYangNeuralNetwork(game)
+        self.neural_net = YinYangNeuralNetwork(game, eval_symmetry=eval_symmetry)
         if os.path.exists(model_path):
             self.neural_net.load_model(model_path)
             logger.info(f"Loaded model from {model_path}")
         else:
             logger.warning(f"No model found at {model_path}, using randomly initialized model")
-        self.mcts = MCTS(game=game, neural_net=self.neural_net, num_simulations=num_simulations, num_threads=num_threads)
+        self.mcts = MCTS(game=game, neural_net=self.neural_net, num_simulations=num_simulations, num_threads=num_threads,
+                         eval_symmetry=eval_symmetry)
         self.root = None
 
     def reset(self):

@@ -56,7 +56,7 @@ class RollingSelfPlay:
 
     def __init__(self, game, state_dict=None, slots=MAX_CONCURRENT_GAMES, num_simulations=800, temperature_threshold=10,
                  dirichlet_alpha=0.3, dirichlet_epsilon=0.25, cpuct=1.0, seed=None, evaluator="nn", search_as_black=True,
-                 device=None, replay_capacity=None):
+                 device=None, replay_capacity=None, eval_symmetry="none"):
         self.game = game
         self.n, self.m = game.getBoardSize()
         self.A = self.n * self.m
@@ -71,7 +71,7 @@ class RollingSelfPlay:
                                   cpuct=cpuct, rule_flags=getattr(game, "rule_flags", 0), search_as_black=search_as_black,
                                   dirichlet_alpha=dirichlet_alpha, dirichlet_epsilon=dirichlet_epsilon,
                                   temperature_threshold=temperature_threshold, seed=seed, state_dict=state_dict,
-                                  replay_capacity=replay_capacity, device=device)
+                                  replay_capacity=replay_capacity, device=device, eval_symmetry=eval_symmetry)
         self.cursor = 0                     # records drained so far
         self.games_requested = 0            # quota handed to the engine so far (exact mode)
         self.games_returned = 0
@@ -137,12 +137,12 @@ class RollingSelfPlay:
 
 def play_games_arrays(game, state_dict, num_games, num_simulations=800, temperature_threshold=10, dirichlet_alpha=0.3,
                       dirichlet_epsilon=0.25, cpuct=1.0, seed=None, evaluator="nn", search_as_black=True, device=None,
-                      max_slots=MAX_CONCURRENT_GAMES):
+                      max_slots=MAX_CONCURRENT_GAMES, eval_symmetry="none"):
     """``num_games`` complete self-play games, all concurrent on the GPU; examples as arrays (RollingSelfPlay.drain)."""
     sp = RollingSelfPlay(game, state_dict, slots=max(1, min(num_games, max_slots)), num_simulations=num_simulations,
                          temperature_threshold=temperature_threshold, dirichlet_alpha=dirichlet_alpha,
                          dirichlet_epsilon=dirichlet_epsilon, cpuct=cpuct, seed=seed, evaluator=evaluator,
-                         search_as_black=search_as_black, device=device)
+                         search_as_black=search_as_black, device=device, eval_symmetry=eval_symmetry)
     try:
         return sp.play(num_games)
     finally:
@@ -288,7 +288,8 @@ def save_example_arrays(filename, ex, n, m, wire="arrays", rule_flags=0):
     return save_examples(filename, examples, n * m, wire)
 
 
-def generate_self_play_data(game, model_path, output_dir, num_games=100, num_workers=1, num_simulations=800, wire="native", file_tag=""):
+def generate_self_play_data(game, model_path, output_dir, num_games=100, num_workers=1, num_simulations=800, wire="native", file_tag="",
+                            eval_symmetry="none"):
     """self_play.py:337-387.  Returns the path of the written .npz (``wire``: see save_examples / save_example_arrays;
     ``file_tag``: suffix that keeps the files of several ranks apart).  num_workers x (num_games // num_workers) games
     (self_play.py:355), all concurrent on the GPU."""
@@ -297,7 +298,7 @@ def generate_self_play_data(game, model_path, output_dir, num_games=100, num_wor
     n, m = game.getBoardSize()
     try:
         net = _load_network(game, model_path)
-        ex = play_games_arrays(game, net.state_dict(), num_workers * games_per_worker, num_simulations)
+        ex = play_games_arrays(game, net.state_dict(), num_workers * games_per_worker, num_simulations, eval_symmetry=eval_symmetry)
     except Exception as e:  # self_play.py:283-286: a failed worker contributes no examples
         logger.error(f"Self-play failed: {e}")
         ex = {"boards": np.zeros((0, n, m), np.int8), "pi": np.zeros((0, n * m)), "z": np.zeros(0)}
@@ -308,7 +309,7 @@ def generate_self_play_data(game, model_path, output_dir, num_games=100, num_wor
 
 
 def generate_self_play_data_distributed(game, model_path, output_dir, num_games=100, num_simulations=800, wire="arrays",
-                                        backend=None):
+                                        backend=None, eval_symmetry="none"):
     """generate_self_play_data for one process per GPU (``torchrun``): every rank plays its contiguous share of the
     ``num_games`` games with its own random streams, the examples are gathered to rank 0 (NCCL all-gather of the record
     tensors; gloo in the CPU tests' plumbing check) and rank 0 writes ONE ``self_play_data_<time>.npz``.  Initialises the
@@ -329,7 +330,7 @@ def generate_self_play_data_distributed(game, model_path, output_dir, num_games=
     dist.broadcast(t, 0)                                              # one base seed for the job, a distinct stream per rank
     seed = yyd.rank_seed(int(t.item()), rank) & 0x7FFFFFFFFFFFFFFF
     if hi > lo:
-        ex = play_games_arrays(game, net.state_dict(), hi - lo, num_simulations, seed=seed)
+        ex = play_games_arrays(game, net.state_dict(), hi - lo, num_simulations, seed=seed, eval_symmetry=eval_symmetry)
     else:
         ex = {"boards": np.zeros((0, n, m), np.int8), "pi": np.zeros((0, n * m)), "z": np.zeros(0), "game": np.zeros(0, np.int32),
               "counts": np.zeros((0, n * m), np.uint16)}
