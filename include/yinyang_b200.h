@@ -274,6 +274,15 @@ int yy_selfplay_set_quota(yy_engine *e, int64_t total_games);
  * by the caller and must outlive the self-play calls. */
 int yy_selfplay_set_random_stream(yy_engine *e, const double *uniforms_dev, const double *noise_dev, int32_t n_games,
                                   int32_t n_plies);
+/* Playout cap randomisation of self-play (yy_selfplay_run / yy_selfplay_advance): each move is a full search (n_sims
+ * simulations, noise as usual, recorded) with probability full_prob -- decided by a hash of (seed, game serial, ply) --
+ * otherwise a fast search (fast_sims simulations, no noise, not recorded).  full_prob = 1 turns it off (the default).
+ * Applies from the next search root each slot prepares; yy_search* ignore it.
+ *   full(s, p) = (mix64(mix64(seed ^ 0x706c61796f757463) ^ ((uint64)(uint32)s << 20 | p)) >> 32) < llround(full_prob 2^32)
+ * A fast move chooses, applies and ends the game exactly as a full one; it adds no replay record (stats: `moves`
+ * counts every search, `examples` the full ones).  YY_ERR_INVALID for full_prob outside [0, 1] or NaN and for fast_sims
+ * outside [1, n_sims]; YY_ERR_STATE with the EXTERNAL evaluator. */
+int yy_selfplay_set_playout_cap(yy_engine *e, double full_prob, int32_t fast_sims);
 
 typedef struct {
   int64_t moves;          /* searches completed                         */

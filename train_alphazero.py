@@ -53,6 +53,12 @@ def parse_args(argv=None):
     p.add_argument("--eval-symmetry", choices=["none", "random", "average"], default="none",
                    help="network evaluation of the search leaves in every mode: as they are (default), in one dihedral form "
                         "of the board hashed from the position and the seed, or averaged over all forms (8x the network FLOPs)")
+    p.add_argument("--full-search-prob", type=float, default=1.0,
+                   help="self-play playout cap randomisation (--mode self-play / train): the share of moves that get the full "
+                        "--simulations search and become training examples; the others get a fast search that only advances "
+                        "the game (default 1: every move)")
+    p.add_argument("--fast-simulations", type=int, default=None,
+                   help="simulations of a fast self-play search when --full-search-prob < 1 (default: --simulations)")
     return p.parse_args(argv)
 
 
@@ -80,7 +86,8 @@ def main(argv=None):
         az = AlphaZero(game=game, model_dir=args.model_dir, data_dir=args.data_dir, num_iterations=args.iterations,
                        num_episodes=args.episodes, num_simulations=args.simulations, num_epochs=args.epochs,
                        num_workers=args.workers, mcts_threads=args.mcts_threads, eval_games=args.arena_games,
-                       batch_size=args.batch_size, lr=args.lr, eval_symmetry=args.eval_symmetry)
+                       batch_size=args.batch_size, lr=args.lr, eval_symmetry=args.eval_symmetry,
+                       full_search_prob=args.full_search_prob, fast_simulations=args.fast_simulations)
         if args.file_loop:
             az.run()                                                     # the reference's loop: data files between the stages
         else:
@@ -105,12 +112,15 @@ def main(argv=None):
             from yinyang_game_alphazero_b200.self_play import generate_self_play_data_distributed
             data_file = generate_self_play_data_distributed(game=game, model_path=model_path, output_dir=args.data_dir,
                                                             num_games=args.episodes, num_simulations=args.simulations,
-                                                            wire=args.replay_wire, eval_symmetry=args.eval_symmetry)
+                                                            wire=args.replay_wire, eval_symmetry=args.eval_symmetry,
+                                                            full_search_prob=args.full_search_prob,
+                                                            fast_simulations=args.fast_simulations)
         else:
             data_file = generate_self_play_data(game=game, model_path=model_path, output_dir=args.data_dir,
                                                 num_games=args.episodes, num_workers=args.workers,
                                                 num_simulations=args.simulations, wire=args.replay_wire,
-                                                eval_symmetry=args.eval_symmetry)
+                                                eval_symmetry=args.eval_symmetry, full_search_prob=args.full_search_prob,
+                                                fast_simulations=args.fast_simulations)
         if data_file:
             logger.info(f"Self-play data generation completed. Data saved to {data_file}")
         return 0

@@ -41,9 +41,11 @@ def _barrier():
 class AlphaZero:
     def __init__(self, game, model_dir="models", data_dir="data", num_iterations=100, num_episodes=100, num_simulations=800,
                  num_epochs=10, temperature_threshold=10, update_threshold=0.6, num_workers=1, mcts_threads=1, eval_games=40,
-                 batch_size=64, lr=0.001, eval_symmetry="none"):
+                 batch_size=64, lr=0.001, eval_symmetry="none", full_search_prob=1.0, fast_simulations=None):
         self.game, self.model_dir, self.data_dir = game, model_dir, data_dir
         self.eval_symmetry = eval_symmetry      # leaf evaluation of the self-play and arena searches (Engine(eval_symmetry=))
+        # playout cap randomisation of self-play (RollingSelfPlay); the arena always searches with num_simulations
+        self.full_search_prob, self.fast_simulations = full_search_prob, fast_simulations
         self.num_iterations, self.num_episodes, self.num_simulations = num_iterations, num_episodes, num_simulations
         self.num_epochs, self.temperature_threshold, self.update_threshold = num_epochs, temperature_threshold, update_threshold
         self.num_workers, self.mcts_threads, self.eval_games = num_workers, mcts_threads, eval_games
@@ -65,7 +67,8 @@ class AlphaZero:
         lo, hi = shard_games(self.num_episodes, self.world, self.rank)
         path = generate_self_play_data(game=self.game, model_path=model_path, output_dir=self.data_dir, num_games=max(1, hi - lo),
                                        num_workers=self.num_workers, num_simulations=self.num_simulations,
-                                       file_tag=f"_r{self.rank}" if self.world > 1 else "", eval_symmetry=self.eval_symmetry)
+                                       file_tag=f"_r{self.rank}" if self.world > 1 else "", eval_symmetry=self.eval_symmetry,
+                                       full_search_prob=self.full_search_prob, fast_simulations=self.fast_simulations)
         _barrier()                                                                  # all data files are on disk
         return path
 
@@ -104,7 +107,8 @@ class AlphaZero:
                           num_simulations=self.num_simulations, num_epochs=self.num_epochs, batch_size=self.batch_size, lr=self.lr,
                           update_threshold=self.update_threshold, eval_games=self.eval_games, num_channels=C, num_res_blocks=B,
                           slots=slots, temperature_threshold=self.temperature_threshold, exact_episodes=exact_episodes,
-                          mcts_threads=self.mcts_threads, state_dict=sd, eval_symmetry=self.eval_symmetry)
+                          mcts_threads=self.mcts_threads, state_dict=sd, eval_symmetry=self.eval_symmetry,
+                          full_search_prob=self.full_search_prob, fast_simulations=self.fast_simulations)
         try:
             return loop.run()
         finally:

@@ -35,6 +35,10 @@ struct EngineDev {
   uint32_t mode_flags;
   int temperature_threshold;
   uint64_t seed;
+  // playout cap randomisation of self-play (yy_selfplay_set_playout_cap): a move is a full search iff
+  // hash(seed, serial, ply) >> 32 < cap_threshold (2^32 = always: the default), otherwise a fast one of fast_sims
+  uint64_t cap_threshold;
+  int fast_sims;
   // nodes
   uint64_t* node_black; uint64_t* node_white;
   int32_t* node_edge_base; int16_t* node_n_edges; int8_t* node_player; uint8_t* node_flags; float* node_value;
@@ -42,6 +46,7 @@ struct EngineDev {
   int32_t* edge_N; float* edge_W; float* edge_P; uint64_t* edge_cmeta; uint8_t* edge_action;
   // per game search state
   int32_t* g_n_nodes; int32_t* g_n_edges; int32_t* g_sims_done;
+  int32_t* g_sim_budget; // simulations the game's current search runs (n_sims, or fast_sims for a fast self-play move)
   int32_t* g_npending;   // leaves waiting for the evaluator; 0 = no search in progress; -1 = search in progress, no leaf this step
   // pending leaf batch (evaluator input), slot = game*K + k: node id, recorded path, state, rules result
   int32_t* leaf_node; int32_t* leaf_path_len; int32_t* leaf_path;
@@ -55,6 +60,7 @@ struct EngineDev {
   // self-play slots
   uint64_t* sp_black; uint64_t* sp_white; int8_t* sp_player; int32_t* sp_step; int32_t* sp_passes; int32_t* sp_serial;
   uint8_t* sp_new_game;
+  uint8_t* sp_full;         // 1 = the slot's current search is a full one: its move is recorded in the replay ring
   int32_t* sp_next_serial;
   // rolling self-play inside the persistent kernel (yy_fused.cu): a slot whose search is complete makes its move and
   // roots the next search at once, independently of the other slots

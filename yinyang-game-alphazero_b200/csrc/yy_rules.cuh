@@ -302,4 +302,11 @@ YY_HD int hashed_form(uint64_t key, uint64_t seed, int rows, int cols) {
   return form_at((int)(mix64(key ^ seed) % (uint64_t)form_count(rows, cols)), rows, cols);
 }
 
+// ---- playout cap randomisation of self-play: the search of game `serial` at ply `ply` is a full one iff this holds
+// (threshold = llround(p_full * 2^32); 2^32 = always, 0 = never).  A pure function of (engine seed, serial, ply).
+YY_HD bool playout_full(uint64_t seed, int serial, int ply, uint64_t threshold) {
+  const uint64_t key = mix64(mix64(seed ^ 0x706c61796f757463ull) ^ (((uint64_t)(uint32_t)serial << 20) | (uint64_t)(uint32_t)ply));
+  return (key >> 32) < threshold;
+}
+
 }  // namespace yy

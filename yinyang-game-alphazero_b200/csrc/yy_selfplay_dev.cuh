@@ -26,16 +26,19 @@ __device__ __forceinline__ int next_game_serial(const EngineDev& e) {
 
 // Top of the play_game loop (self_play.py:91-125): new game if needed, pass / double-pass handling, then the root of
 // the next search.  search player = 1 always under YY_MODE_SEARCH_AS_BLACK (self_play.py:99,135-137).
-// Returns false when the slot needs a new game and the quota is used up (the slot idles).
+// Playout cap: the search is a full one (n_sims, noise at ply 0, recorded) or a fast one (fast_sims, no noise, not
+// recorded) as playout_full decides for (seed, serial, ply).
+// Returns the simulation budget of the search, or -1 when the slot needs a new game and the quota is used up (the slot
+// idles).
 template <int NW>
-__device__ __forceinline__ bool sp_prepare_one(const EngineDev& e, const Geo<NW>& g, int gi) {
+__device__ __forceinline__ int sp_prepare_one(const EngineDev& e, const Geo<NW>& g, int gi) {
   BB<NW> b = load_bb<NW>(e.sp_black, gi, e.W), w = load_bb<NW>(e.sp_white, gi, e.W);
   int player = e.sp_player[gi], step = e.sp_step[gi], passes = e.sp_passes[gi];
   int sp = 1;
   for (;;) {
     if (e.sp_new_game[gi]) {
       const int serial = next_game_serial(e);
-      if (serial < 0) { e.sp_serial[gi] = -1; return false; }
+      if (serial < 0) { e.sp_serial[gi] = -1; return -1; }
       b = bb_zero<NW>(); w = bb_zero<NW>(); player = 1; step = 0; passes = 0;
       e.sp_serial[gi] = serial;
       e.sp_new_game[gi] = 0;
@@ -56,8 +59,10 @@ __device__ __forceinline__ bool sp_prepare_one(const EngineDev& e, const Geo<NW>
   e.sp_player[gi] = (int8_t)player; e.sp_step[gi] = step; e.sp_passes[gi] = passes;
   store_bb<NW>(e.root_black, gi, e.W, b); store_bb<NW>(e.root_white, gi, e.W, w);
   e.root_player[gi] = (int8_t)sp;
-  e.noise_mask[gi] = (step == 0 && e.eps > 0.0) ? 1 : 0;  // add_noise = (step == 0), self_play.py:131
-  return true;
+  const bool full = playout_full(e.seed, e.sp_serial[gi], step, e.cap_threshold);
+  e.sp_full[gi] = full ? 1 : 0;
+  e.noise_mask[gi] = (full && step == 0 && e.eps > 0.0) ? 1 : 0;  // add_noise = (step == 0), self_play.py:131
+  return full ? e.n_sims : e.fast_sims;
 }
 
 __device__ inline double gamma_sample(Philox& rng, double a) {
@@ -107,20 +112,24 @@ __device__ __forceinline__ void sp_move_one(const EngineDev& e, const Geo<NW>& g
   int player = e.sp_player[gi], step = e.sp_step[gi];
   const int serial = e.sp_serial[gi];
   const int base = e.node_edge_base[nb], cnt = (e.node_flags[nb] & NODE_EXPANDED) ? e.node_n_edges[nb] : 0;
-  // example record (board before the move, visit counts; pi = counts/sum on the host in float64)
-  unsigned long long slot64 = atomicAdd(&e.stats->examples, 1ull);
-  long long slot = (long long)(slot64 % (unsigned long long)e.replay_cap);
-  store_bb<NW>(e.rp_black, slot, e.W, b); store_bb<NW>(e.rp_white, slot, e.W, w);
-  uint16_t* rc = e.rp_counts + slot * e.A;
-  for (int a = 0; a < e.A; ++a) rc[a] = 0;
+  // example record (board before the move, visit counts; pi = counts/sum on the host in float64) -- full searches only:
+  // a fast search of the playout cap only advances the game
+  uint16_t* rc = nullptr;
+  if (e.sp_full[gi]) {
+    unsigned long long slot64 = atomicAdd(&e.stats->examples, 1ull);
+    long long slot = (long long)(slot64 % (unsigned long long)e.replay_cap);
+    store_bb<NW>(e.rp_black, slot, e.W, b); store_bb<NW>(e.rp_white, slot, e.W, w);
+    rc = e.rp_counts + slot * e.A;
+    for (int a = 0; a < e.A; ++a) rc[a] = 0;
+    e.rp_serial[slot] = serial; e.rp_ply[slot] = (int16_t)step; e.rp_player[slot] = (int8_t)player;
+  }
   long long total = 0; int maxn = -1, nmax = 0;
   for (int k = 0; k < cnt; ++k) {
     int n = e.edge_N[eb + base + k];
-    rc[e.edge_action[eb + base + k]] = (uint16_t)(n > 65535 ? 65535 : n);
+    if (rc) rc[e.edge_action[eb + base + k]] = (uint16_t)(n > 65535 ? 65535 : n);
     total += n;
     if (n > maxn) { maxn = n; nmax = 1; } else if (n == maxn) ++nmax;
   }
-  e.rp_serial[slot] = serial; e.rp_ply[slot] = (int16_t)step; e.rp_player[slot] = (int8_t)player;
   // one uniform draw per move: the recorded stream when there is one, else Philox keyed by (seed, game, ply)
   double u;
   if (e.hook_uniform && serial >= 0 && serial < e.hook_games && step < e.hook_plies) u = e.hook_uniform[(long long)serial * e.hook_plies + step];
@@ -150,13 +159,14 @@ __device__ __forceinline__ void sp_move_one(const EngineDev& e, const Geo<NW>& g
   if (code != 0) finish_game(e, gi, code);
 }
 
-// MCTS.search prologue (mcts.py:288-292) for one game, by its warp: fresh tree, root = node 0 = the pending leaf.
+// MCTS.search prologue (mcts.py:288-292) for one game, by its warp: fresh tree, root = node 0 = the pending leaf; the
+// search runs `budget` simulations.
 template <int NW>
-__device__ __forceinline__ void tree_root_game(const EngineDev& e, const Geo<NW>& g, int gi, int lane) {
+__device__ __forceinline__ void tree_root_game(const EngineDev& e, const Geo<NW>& g, int gi, int lane, int budget) {
   BB<NW> b = load_bb<NW>(e.root_black, gi, e.W) & g.full, w = load_bb<NW>(e.root_white, gi, e.W) & g.full;
   int player = e.root_player[gi] == 1 ? 1 : -1;
   if (lane == 0) {
-    e.g_n_nodes[gi] = 1; e.g_n_edges[gi] = 0; e.g_sims_done[gi] = 0; e.g_npending[gi] = 1;
+    e.g_n_nodes[gi] = 1; e.g_n_edges[gi] = 0; e.g_sims_done[gi] = 0; e.g_npending[gi] = 1; e.g_sim_budget[gi] = budget;
     for (int k = 1; k < e.K; ++k) e.leaf_active[gi * e.K + k] = 0;
   }
   publish_leaf<NW>(e, g, gi, lane, gi * e.K, 0, b, w, player, 0);
@@ -169,7 +179,7 @@ __device__ __forceinline__ void tree_root_game(const EngineDev& e, const Geo<NW>
 // its code out of the persistent kernel's hot loops, and the kernel's parameter structs stay in constant memory.
 template <int NW>
 __device__ __noinline__ void sp_advance_game(const EngineDev e, const Geo<NW> g, int gi, int lane) {
-  int go = 0;
+  int budget = -1;
   if (lane == 0) {
     int left = e.sp_moves_left[gi];
     if (e.sp_phase[gi] && left > 0) {
@@ -177,12 +187,15 @@ __device__ __noinline__ void sp_advance_game(const EngineDev e, const Geo<NW> g,
       e.sp_phase[gi] = 0;
       if (left != kMovesUnlimited) e.sp_moves_left[gi] = --left;
     }
-    if (!e.sp_phase[gi] && left > 0 && sp_prepare_one<NW>(e, g, gi)) { sp_noise_one<NW>(e, g, gi); go = 1; }
+    if (!e.sp_phase[gi] && left > 0) {
+      budget = sp_prepare_one<NW>(e, g, gi);
+      if (budget >= 0) sp_noise_one<NW>(e, g, gi);
+    }
   }
-  go = __shfl_sync(kFull, go, 0);
-  if (!go) return;
+  budget = __shfl_sync(kFull, budget, 0);
+  if (budget < 0) return;
   __syncwarp();
-  tree_root_game<NW>(e, g, gi, lane);
+  tree_root_game<NW>(e, g, gi, lane, budget);
   if (lane == 0) e.sp_phase[gi] = 1;
   __syncwarp();
 }

@@ -23,11 +23,13 @@ namespace yy {
 constexpr int kTreeBlock = 128;  // 4 games per CTA
 
 // MCTS.search prologue (mcts.py:288-292): fresh tree per game, root = node 0, pending leaf = root (slot g*K).
+// A plain search runs n_sims simulations; the lock-step self-play driver (`prepared`) keeps the budget sp_prepare_kernel
+// chose (playout cap).
 template <int NW>
-__global__ void __launch_bounds__(kTreeBlock) tree_root_kernel(EngineDev e, Geo<NW> g) {
+__global__ void __launch_bounds__(kTreeBlock) tree_root_kernel(EngineDev e, Geo<NW> g, int prepared) {
   int gi = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
   if (gi >= e.n_games) return;
-  tree_root_game<NW>(e, g, gi, lane);
+  tree_root_game<NW>(e, g, gi, lane, prepared ? e.g_sim_budget[gi] : e.n_sims);
   if (lane == 0) e.sp_phase[gi] = 0;      // the tree no longer belongs to a rolling self-play search (sp_advance_game)
   if (gi == 0 && lane == 0) { e.active_count[0] = e.n_games; e.active_count[1] = 0; }
 }
@@ -78,7 +80,8 @@ template <int NW>
 __global__ void __launch_bounds__(128) sp_prepare_kernel(EngineDev e, Geo<NW> g) {
   int gi = blockIdx.x * blockDim.x + threadIdx.x;
   if (gi >= e.n_games) return;
-  sp_prepare_one<NW>(e, g, gi);
+  const int budget = sp_prepare_one<NW>(e, g, gi);
+  e.g_sim_budget[gi] = budget >= 0 ? budget : e.n_sims;     // read by the root kernel of this move's search
 }
 template <int NW>
 __global__ void __launch_bounds__(128) sp_noise_kernel(EngineDev e, Geo<NW> g) {
@@ -149,6 +152,7 @@ static void carve(const yy_engine_config& c, Carver& k, EngineDev& d) {
   d.edge_N = k.take<int32_t>(G * EC); d.edge_W = k.take<float>(G * EC); d.edge_P = k.take<float>(G * EC);
   d.edge_cmeta = k.take<uint64_t>(G * EC); d.edge_action = k.take<uint8_t>(G * EC);
   d.g_n_nodes = k.take<int32_t>(G); d.g_n_edges = k.take<int32_t>(G); d.g_sims_done = k.take<int32_t>(G);
+  d.g_sim_budget = k.take<int32_t>(G);
   d.K = c.leaves_per_step; d.n_slots = c.n_games * c.leaves_per_step;
   const size_t S = (size_t)d.n_slots;
   d.g_npending = k.take<int32_t>(G);
@@ -160,7 +164,7 @@ static void carve(const yy_engine_config& c, Carver& k, EngineDev& d) {
   d.noise = k.take<double>(G * A); d.noise_mask = k.take<uint8_t>(G);
   d.sp_black = k.take<uint64_t>(G * W); d.sp_white = k.take<uint64_t>(G * W); d.sp_player = k.take<int8_t>(G);
   d.sp_step = k.take<int32_t>(G); d.sp_passes = k.take<int32_t>(G); d.sp_serial = k.take<int32_t>(G);
-  d.sp_new_game = k.take<uint8_t>(G); d.sp_next_serial = k.take<int32_t>(1);
+  d.sp_new_game = k.take<uint8_t>(G); d.sp_full = k.take<uint8_t>(G); d.sp_next_serial = k.take<int32_t>(1);
   d.sp_phase = k.take<uint8_t>(G); d.sp_moves_left = k.take<int32_t>(G); d.act_list = k.take<int32_t>(G);
   d.game_quota = -1; d.hook_uniform = nullptr; d.hook_noise = nullptr; d.hook_games = 0; d.hook_plies = 0;
   const size_t RC = (size_t)c.replay_capacity;
@@ -190,9 +194,9 @@ namespace {
 inline unsigned warp_grid(int n_games) { return (unsigned)(((long long)n_games * 32 + kTreeBlock - 1) / kTreeBlock); }
 inline unsigned thread_grid(int n, int block) { return (unsigned)((n + block - 1) / block); }
 
-int launch_root(yy_engine* e, cudaStream_t s) {
+int launch_root(yy_engine* e, cudaStream_t s, bool prepared = false) {
   YY_DISPATCH_NW(e->dev.A, tree_root_kernel<NW><<<warp_grid(e->dev.n_games), kTreeBlock, 0, s>>>(
-      e->dev, make_geo<NW>(e->cfg.rows, e->cfg.cols, e->cfg.rule_flags)));
+      e->dev, make_geo<NW>(e->cfg.rows, e->cfg.cols, e->cfg.rule_flags), prepared ? 1 : 0));
   YY_LAUNCH_CHECK();
   e->step_parity = 0;   // root wrote [0] = n_games, [1] = 0; the first step counts into [1]
   return YY_OK;
@@ -235,9 +239,10 @@ int run_evaluator(yy_engine* e, cudaStream_t s) {
                           engine_forms(e), s);
   return set_error(YY_ERR_STATE, "external evaluator: use yy_search_begin / yy_search_advance");
 }
-// full search over the roots already stored in dev.root_* (noise pointers already set in dev)
-int search_core(yy_engine* e, cudaStream_t s) {
-  int rc = launch_root(e, s); if (rc) return rc;
+// full search over the roots already stored in dev.root_* (noise pointers already set in dev); `prepared`: the
+// lock-step self-play driver's search, with the simulation budget sp_prepare_kernel chose per game
+int search_core(yy_engine* e, cudaStream_t s, bool prepared = false) {
+  int rc = launch_root(e, s, prepared); if (rc) return rc;
   if (e->cfg.leaves_per_step <= 1 && !(e->cfg.mode_flags & YY_MODE_STEP_KERNELS) && e->cfg.evaluator != YY_EVAL_EXTERNAL) {
     // the whole search in ONE persistent kernel: every CTA owns a run of games from the first to the last simulation
     // (the launch ends as soon as no game has work left; a game advances by at least one simulation every two steps)
@@ -314,6 +319,7 @@ yy_engine* yy_engine_create(const yy_engine_config* cfg, void* workspace, int64_
   e->dev.keep_f32 = (float)(1.0 - (double)c.dirichlet_epsilon);
   e->dev.evaluator = c.evaluator; e->dev.mode_flags = c.mode_flags; e->dev.temperature_threshold = c.temperature_threshold;
   e->dev.seed = c.seed;
+  e->dev.cap_threshold = 1ull << 32; e->dev.fast_sims = c.n_sims;      // playout cap off: every move a full search
   e->dev.max_descents = c.descents_per_step == 0 ? 4 : (c.descents_per_step < 0 ? 0 : c.descents_per_step);
   size_t off = (k.off + 255) & ~(size_t)255;
   if (nn_init(e->nn, c, (char*)workspace + off) != YY_OK) { delete e; return nullptr; }
@@ -488,7 +494,7 @@ int yy_selfplay_run(yy_engine* e, int32_t n_moves, void* stream) {
     YY_LAUNCH_CHECK();
     YY_DISPATCH_NW(e->dev.A, sp_noise_kernel<NW><<<grid, 128, 0, s>>>(e->dev, make_geo<NW>(e->cfg.rows, e->cfg.cols, e->cfg.rule_flags)));
     YY_LAUNCH_CHECK();
-    int rc = search_core(e, s); if (rc) return rc;
+    int rc = search_core(e, s, true); if (rc) return rc;
     YY_DISPATCH_NW(e->dev.A, sp_move_kernel<NW><<<grid, 128, 0, s>>>(e->dev, make_geo<NW>(e->cfg.rows, e->cfg.cols, e->cfg.rule_flags)));
     YY_LAUNCH_CHECK();
   }
@@ -505,6 +511,17 @@ int yy_selfplay_advance(yy_engine* e, int64_t iterations, void* stream) {
 int yy_selfplay_set_quota(yy_engine* e, int64_t total_games) {
   if (!e) return set_error(YY_ERR_INVALID, "null engine");
   e->dev.game_quota = total_games < 0 ? -1 : (long long)total_games;
+  return YY_OK;
+}
+
+int yy_selfplay_set_playout_cap(yy_engine* e, double full_prob, int32_t fast_sims) {
+  if (!e) return set_error(YY_ERR_INVALID, "null engine");
+  if (e->cfg.evaluator == YY_EVAL_EXTERNAL) return set_error(YY_ERR_STATE, "self-play needs the STUB or NN evaluator");
+  if (!(full_prob >= 0.0 && full_prob <= 1.0)) return set_error(YY_ERR_INVALID, "full_prob must be in [0, 1]");
+  if (fast_sims < 1 || fast_sims > e->cfg.n_sims)
+    return set_error(YY_ERR_INVALID, "fast_sims must be in [1, n_sims = %d], not %d", e->cfg.n_sims, (int)fast_sims);
+  e->dev.cap_threshold = (uint64_t)llround(full_prob * 4294967296.0);
+  e->dev.fast_sims = fast_sims;
   return YY_OK;
 }
 

@@ -155,7 +155,8 @@ __device__ __forceinline__ int tree_step_game(const EngineDev& e, const Geo<NW>&
   const long long nb = (long long)gi * e.max_nodes;
   const long long eb = (long long)gi * e.edges_cap;
   const bool multi = e.K > 1;
-  int sims_done = e.g_sims_done[gi];
+  // simulations this search still has to run: its budget (n_sims; fast_sims for a fast self-play search) minus those done
+  int left = e.g_sim_budget[gi] - e.g_sims_done[gi];
   int sims_here = 0, evals_here = 0, deepest = 0;
 
   // ---------------------------------------------------------------- (1) expand + backup
@@ -164,13 +165,13 @@ __device__ __forceinline__ int tree_step_game(const EngineDev& e, const Geo<NW>&
     const int slot = gi * e.K + k;
     const bool is_root = e.leaf_node[slot] == 0;
     expand_and_backup<NW>(e, g, gi, lane, slot, nb, eb, multi);
-    if (!is_root) { ++sims_done; ++sims_here; }
+    if (!is_root) { --left; ++sims_here; }
   }
 
   // ---------------------------------------------------------------- (2) select
   int np = 0, descents = 0;
   bool blocked = false;
-  while (sims_done + np < e.n_sims && np < e.K && !blocked) {
+  while (np < left && np < e.K && !blocked) {
     if (max_descents > 0 && descents++ >= max_descents) break;
     const int slot = gi * e.K + np;
     int32_t* path = e.leaf_path + (long long)slot * e.max_depth;
@@ -182,7 +183,7 @@ __device__ __forceinline__ int tree_step_game(const EngineDev& e, const Geo<NW>&
       if (fl & (NODE_TERMINAL | NODE_NOCHILD)) {   // revisited terminal (mcts.py:365-367) / child-less node
         __syncwarp();                              // path[] written by lane 0 above
         backup_path(e, path, eb, depth, e.node_value[nb + node], lane, false);
-        ++sims_done; ++sims_here;
+        --left; ++sims_here;
         __syncwarp();
         break;
       }
@@ -249,9 +250,9 @@ __device__ __forceinline__ int tree_step_game(const EngineDev& e, const Geo<NW>&
     }
   }
   __syncwarp();
-  const bool selecting = np == 0 && !blocked && sims_done < e.n_sims;     // stopped by max_descents
+  const bool selecting = np == 0 && !blocked && left > 0;                 // stopped by max_descents
   if (lane == 0) {
-    e.g_sims_done[gi] = sims_done;
+    e.g_sims_done[gi] += sims_here;
     e.g_npending[gi] = selecting ? -1 : np;
     if (np && pending_counter) atomicAdd(pending_counter, np);
     if (sims_here) atomicAdd(&e.stats->sims, (unsigned long long)sims_here);

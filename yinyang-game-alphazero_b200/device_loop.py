@@ -65,7 +65,8 @@ class DeviceSelfPlay:
     """Rolling self-play whose finished games stay on the device (engine replay ring -> device tensors)."""
 
     def __init__(self, game, state_dict, slots=4096, num_simulations=800, temperature_threshold=10, dirichlet_alpha=0.3,
-                 dirichlet_epsilon=0.25, cpuct=1.0, seed=0, evaluator="nn", device=None, eval_symmetry="none"):
+                 dirichlet_epsilon=0.25, cpuct=1.0, seed=0, evaluator="nn", device=None, eval_symmetry="none", full_search_prob=1.0,
+                 fast_simulations=None):
         self.n, self.m = game.getBoardSize()
         self.A, self.slots, self.sims = self.n * self.m, int(slots), int(num_simulations)
         self.eng = _engine.Engine(rows=self.n, cols=self.m, n_games=self.slots, n_sims=self.sims, evaluator=evaluator, cpuct=cpuct,
@@ -73,6 +74,8 @@ class DeviceSelfPlay:
                                   dirichlet_epsilon=dirichlet_epsilon, temperature_threshold=temperature_threshold, seed=seed,
                                   state_dict=state_dict, replay_capacity=self.slots * (2 * self.A + 8) + 4096, device=device,
                                   eval_symmetry=eval_symmetry)
+        if full_search_prob != 1.0 or fast_simulations is not None:      # playout cap: only full searches are recorded
+            self.eng.selfplay_set_playout_cap(full_search_prob, fast_simulations)
         self.cursor, self._pend = 0, None
         self.games_done = 0
 
@@ -124,7 +127,7 @@ class DeviceLoop:
     def __init__(self, game, model_dir="models", num_iterations=100, num_episodes=100, num_simulations=800, num_epochs=10,
                  batch_size=64, lr=0.001, weight_decay=1e-4, sample_size=10000, queue_size=500000, update_threshold=0.6, eval_games=40,
                  num_channels=128, num_res_blocks=10, slots=4096, temperature_threshold=10, exact_episodes=False, save_files=True,
-                 seed=0, mcts_threads=1, state_dict=None, eval_symmetry="none"):
+                 seed=0, mcts_threads=1, state_dict=None, eval_symmetry="none", full_search_prob=1.0, fast_simulations=None):
         self.game, self.model_dir = game, model_dir
         self.eval_symmetry = eval_symmetry
         self.num_iterations, self.num_episodes, self.num_simulations, self.num_epochs = num_iterations, num_episodes, num_simulations, num_epochs
@@ -143,7 +146,8 @@ class DeviceLoop:
         self.episodes_per_rank = share
         self.selfplay = DeviceSelfPlay(game, self.best_sd, slots=max(1, min(slots, share)), num_simulations=num_simulations,
                                        temperature_threshold=temperature_threshold, seed=seed * 1000003 + self.rank,
-                                       eval_symmetry=eval_symmetry)
+                                       eval_symmetry=eval_symmetry, full_search_prob=full_search_prob,
+                                       fast_simulations=fast_simulations)
         self.buffer = DeviceReplayBuffer(self.selfplay.eng.W, n * m, queue_size)
         self.gen = torch.Generator(device="cuda")
         self.gen.manual_seed(seed * 7919 + self.rank)

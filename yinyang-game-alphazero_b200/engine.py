@@ -525,6 +525,14 @@ class Engine:
         """At most total_games games are started since the last reset (None / negative: unlimited)."""
         _lib.check(self.L.yy_selfplay_set_quota(self.handle, -1 if total_games is None else int(total_games)))
 
+    def selfplay_set_playout_cap(self, full_prob=1.0, fast_sims=None):
+        """Playout cap randomisation of self-play (yy_selfplay_set_playout_cap): each move is a full search (n_sims, noise at
+        ply 0, recorded) with probability full_prob -- a hash of (seed, game serial, ply) decides -- otherwise a fast search
+        of fast_sims simulations (None: n_sims) that adds no noise and no replay record.  full_prob=1 turns it off.  Applies
+        from the next search root each slot prepares; search() ignores it."""
+        fast = self.n_sims if fast_sims is None else int(fast_sims)
+        _lib.check(self.L.yy_selfplay_set_playout_cap(self.handle, float(full_prob), fast))
+
     def selfplay_set_random_stream(self, uniforms=None, noise=None):
         """Recorded random stream (yy_selfplay_set_random_stream): uniforms float64[n_games, n_plies], noise float64[n_games, A]
         (numpy or device tensors).  None, None restores Philox."""

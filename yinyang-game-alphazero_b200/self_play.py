@@ -52,11 +52,15 @@ class RollingSelfPlay:
     the host and returns the examples of every game that has FINISHED since (arrays, no per-example Python objects);
     ``play(num_games)`` runs until that many more games are complete.  With ``keep_warm=True`` the other slots keep
     their games in flight for the next call (a rolling generation has no tail); otherwise exactly ``num_games`` games
-    are started (game quota) and the slots idle when they are done."""
+    are started (game quota) and the slots idle when they are done.
+
+    ``full_search_prob`` < 1 turns on playout cap randomisation (Engine.selfplay_set_playout_cap): only that share of
+    the moves gets the full ``num_simulations`` search and a record; the others get a fast search of
+    ``fast_simulations`` (None: num_simulations) that only advances the game."""
 
     def __init__(self, game, state_dict=None, slots=MAX_CONCURRENT_GAMES, num_simulations=800, temperature_threshold=10,
                  dirichlet_alpha=0.3, dirichlet_epsilon=0.25, cpuct=1.0, seed=None, evaluator="nn", search_as_black=True,
-                 device=None, replay_capacity=None, eval_symmetry="none"):
+                 device=None, replay_capacity=None, eval_symmetry="none", full_search_prob=1.0, fast_simulations=None):
         self.game = game
         self.n, self.m = game.getBoardSize()
         self.A = self.n * self.m
@@ -72,6 +76,8 @@ class RollingSelfPlay:
                                   dirichlet_alpha=dirichlet_alpha, dirichlet_epsilon=dirichlet_epsilon,
                                   temperature_threshold=temperature_threshold, seed=seed, state_dict=state_dict,
                                   replay_capacity=replay_capacity, device=device, eval_symmetry=eval_symmetry)
+        if full_search_prob != 1.0 or fast_simulations is not None:
+            self.eng.selfplay_set_playout_cap(full_search_prob, fast_simulations)
         self.cursor = 0                     # records drained so far
         self.games_requested = 0            # quota handed to the engine so far (exact mode)
         self.games_returned = 0
@@ -90,7 +96,8 @@ class RollingSelfPlay:
 
     def drain(self):
         """-> dict(boards int8[E,n,m], pi float64[E,A], z float64[E], game int32[E], ply int16[E], player int8[E],
-        counts uint16[E,A]) of the games finished since the last call, sorted by (game, ply); E may be 0."""
+        counts uint16[E,A]) of the games finished since the last call, sorted by (game, ply); E may be 0.  With the
+        playout cap on, a finished game may have no record at all: finished games are counted by the engine."""
         eng = self.eng
         st = self._stats = eng.stats()
         if st.examples - self.cursor > eng.replay_capacity:
@@ -111,7 +118,7 @@ class RollingSelfPlay:
         out = {"boards": bitboard.unpack_boards(new["black"][idx], new["white"][idx], self.n, self.m), "pi": pi,
                "z": _engine.result_from_code(code[idx]), "game": new["game_serial"][idx], "ply": new["ply"][idx],
                "player": new["player"][idx], "counts": counts}
-        self.games_returned += len(np.unique(out["game"]))
+        self.games_returned = st.games_finished
         return out
 
     def play(self, num_games, keep_warm=False, poll_iterations=None):
@@ -137,12 +144,14 @@ class RollingSelfPlay:
 
 def play_games_arrays(game, state_dict, num_games, num_simulations=800, temperature_threshold=10, dirichlet_alpha=0.3,
                       dirichlet_epsilon=0.25, cpuct=1.0, seed=None, evaluator="nn", search_as_black=True, device=None,
-                      max_slots=MAX_CONCURRENT_GAMES, eval_symmetry="none"):
-    """``num_games`` complete self-play games, all concurrent on the GPU; examples as arrays (RollingSelfPlay.drain)."""
+                      max_slots=MAX_CONCURRENT_GAMES, eval_symmetry="none", full_search_prob=1.0, fast_simulations=None):
+    """``num_games`` complete self-play games, all concurrent on the GPU; examples as arrays (RollingSelfPlay.drain).
+    ``full_search_prob`` / ``fast_simulations``: playout cap randomisation (RollingSelfPlay)."""
     sp = RollingSelfPlay(game, state_dict, slots=max(1, min(num_games, max_slots)), num_simulations=num_simulations,
                          temperature_threshold=temperature_threshold, dirichlet_alpha=dirichlet_alpha,
                          dirichlet_epsilon=dirichlet_epsilon, cpuct=cpuct, seed=seed, evaluator=evaluator,
-                         search_as_black=search_as_black, device=device, eval_symmetry=eval_symmetry)
+                         search_as_black=search_as_black, device=device, eval_symmetry=eval_symmetry,
+                         full_search_prob=full_search_prob, fast_simulations=fast_simulations)
     try:
         return sp.play(num_games)
     finally:
@@ -151,13 +160,15 @@ def play_games_arrays(game, state_dict, num_games, num_simulations=800, temperat
 
 def play_games(game, state_dict, num_games, num_simulations=800, temperature_threshold=10, dirichlet_alpha=0.3,
                dirichlet_epsilon=0.25, cpuct=1.0, seed=None, evaluator="nn", search_as_black=True, max_moves=None,
-               device=None):
+               device=None, full_search_prob=1.0, fast_simulations=None):
     """Plays ``num_games`` complete self-play games concurrently.  Returns a list (one entry per game, in game
     order) of example lists ``[(YinYangLogic, pi float64[A], z float), ...]`` -- the reference's per-game return value
-    (self_play.py:72-192); ``play_games_arrays`` is the same without the per-example objects."""
+    (self_play.py:72-192); ``play_games_arrays`` is the same without the per-example objects.  With the playout cap on
+    (``full_search_prob`` < 1) a game's list holds its full-search moves only, and may be empty."""
     n, m = game.getBoardSize()
     ex = play_games_arrays(game, state_dict, num_games, num_simulations, temperature_threshold, dirichlet_alpha,
-                           dirichlet_epsilon, cpuct, seed, evaluator, search_as_black, device)
+                           dirichlet_epsilon, cpuct, seed, evaluator, search_as_black, device,
+                           full_search_prob=full_search_prob, fast_simulations=fast_simulations)
     games = [[] for _ in range(num_games)]
     rule_flags = getattr(game, "rule_flags", 0)
     for i in range(len(ex["z"])):
@@ -289,16 +300,18 @@ def save_example_arrays(filename, ex, n, m, wire="arrays", rule_flags=0):
 
 
 def generate_self_play_data(game, model_path, output_dir, num_games=100, num_workers=1, num_simulations=800, wire="native", file_tag="",
-                            eval_symmetry="none"):
+                            eval_symmetry="none", full_search_prob=1.0, fast_simulations=None):
     """self_play.py:337-387.  Returns the path of the written .npz (``wire``: see save_examples / save_example_arrays;
     ``file_tag``: suffix that keeps the files of several ranks apart).  num_workers x (num_games // num_workers) games
-    (self_play.py:355), all concurrent on the GPU."""
+    (self_play.py:355), all concurrent on the GPU.  ``full_search_prob`` / ``fast_simulations``: playout cap randomisation
+    (RollingSelfPlay)."""
     os.makedirs(output_dir, exist_ok=True)
     games_per_worker = max(1, num_games // num_workers)          # self_play.py:355
     n, m = game.getBoardSize()
     try:
         net = _load_network(game, model_path)
-        ex = play_games_arrays(game, net.state_dict(), num_workers * games_per_worker, num_simulations, eval_symmetry=eval_symmetry)
+        ex = play_games_arrays(game, net.state_dict(), num_workers * games_per_worker, num_simulations, eval_symmetry=eval_symmetry,
+                               full_search_prob=full_search_prob, fast_simulations=fast_simulations)
     except Exception as e:  # self_play.py:283-286: a failed worker contributes no examples
         logger.error(f"Self-play failed: {e}")
         ex = {"boards": np.zeros((0, n, m), np.int8), "pi": np.zeros((0, n * m)), "z": np.zeros(0)}
@@ -309,7 +322,7 @@ def generate_self_play_data(game, model_path, output_dir, num_games=100, num_wor
 
 
 def generate_self_play_data_distributed(game, model_path, output_dir, num_games=100, num_simulations=800, wire="arrays",
-                                        backend=None, eval_symmetry="none"):
+                                        backend=None, eval_symmetry="none", full_search_prob=1.0, fast_simulations=None):
     """generate_self_play_data for one process per GPU (``torchrun``): every rank plays its contiguous share of the
     ``num_games`` games with its own random streams, the examples are gathered to rank 0 (NCCL all-gather of the record
     tensors; gloo in the CPU tests' plumbing check) and rank 0 writes ONE ``self_play_data_<time>.npz``.  Initialises the
@@ -330,7 +343,8 @@ def generate_self_play_data_distributed(game, model_path, output_dir, num_games=
     dist.broadcast(t, 0)                                              # one base seed for the job, a distinct stream per rank
     seed = yyd.rank_seed(int(t.item()), rank) & 0x7FFFFFFFFFFFFFFF
     if hi > lo:
-        ex = play_games_arrays(game, net.state_dict(), hi - lo, num_simulations, seed=seed, eval_symmetry=eval_symmetry)
+        ex = play_games_arrays(game, net.state_dict(), hi - lo, num_simulations, seed=seed, eval_symmetry=eval_symmetry,
+                               full_search_prob=full_search_prob, fast_simulations=fast_simulations)
     else:
         ex = {"boards": np.zeros((0, n, m), np.int8), "pi": np.zeros((0, n * m)), "z": np.zeros(0), "game": np.zeros(0, np.int32),
               "counts": np.zeros((0, n * m), np.uint16)}
