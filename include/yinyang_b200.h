@@ -284,6 +284,25 @@ int yy_selfplay_set_random_stream(yy_engine *e, const double *uniforms_dev, cons
  * outside [1, n_sims]; YY_ERR_STATE with the EXTERNAL evaluator. */
 int yy_selfplay_set_playout_cap(yy_engine *e, double full_prob, int32_t fast_sims);
 
+/* AlphaZero.evaluate (alphazero.py:176-219) for n_games / 2 games on the persistent kernel, both models in one launch.
+ * Model A is the image loaded with yy_engine_load_weights, model B the image weights_b_dev (bytes must equal
+ * yy_nn_weight_bytes of the engine's network; 256-byte aligned).  Slot j searches for model A and slot G + j for model B
+ * in game j (G = n_games / 2); the two halves of the grid run concurrently.  Game j starts from start_black/white_dev[j]
+ * with start_player_dev[j] to move; model A plays black iff a_plays_black_dev[j] != 0.  Every move is
+ * select_action(temperature = 0) of a search without noise: the argmax of the root visit counts, lowest action on ties,
+ * action 0 when the root has no children; an illegal action is a silent no-op and the turn passes (yy_step).  A game
+ * ends when yy_ended for the next player is nonzero or after max_plies plies; a start position that is already over
+ * ends it with 0 plies.  Outputs: out_code_dev int8[G] = YY_RESULT_* from the perspective of the player to move after
+ * the last move (0 when the ply cap ended the game), out_plies_dev int32[G].  Each game is the exact sequential search;
+ * results do not depend on G or on the slot.  The call runs every game to completion (launches of n_sims + 1 evaluation
+ * steps; the host reads the count of finished games once per launch).  It uses the self-play slots and leaves them
+ * reset (yy_selfplay_reset).  YY_ERR_STATE for the STUB / EXTERNAL evaluators, YY_MODE_STEP_KERNELS and
+ * leaves_per_step > 1; YY_ERR_INVALID for an odd n_games, a wrong image size and max_plies < 1; YY_ERR_CAPACITY when a
+ * tree overflows. */
+int yy_arena_run(yy_engine *e, const void *weights_b_dev, int64_t bytes, const uint64_t *start_black_dev,
+                 const uint64_t *start_white_dev, const int8_t *start_player_dev, const uint8_t *a_plays_black_dev,
+                 int32_t max_plies, int8_t *out_code_dev, int32_t *out_plies_dev, void *stream);
+
 typedef struct {
   int64_t moves;          /* searches completed                         */
   int64_t evals;          /* leaf evaluations requested                 */

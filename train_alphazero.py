@@ -59,6 +59,9 @@ def parse_args(argv=None):
                         "the game (default 1: every move)")
     p.add_argument("--fast-simulations", type=int, default=None,
                    help="simulations of a fast self-play search when --full-search-prob < 1 (default: --simulations)")
+    p.add_argument("--arena-opening-plies", type=int, default=0,
+                   help="--mode train: start the current-vs-best games from paired random openings of this many plies (each "
+                        "opening played once with either model as black); default 0: every game from the empty board")
     return p.parse_args(argv)
 
 
@@ -87,7 +90,8 @@ def main(argv=None):
                        num_episodes=args.episodes, num_simulations=args.simulations, num_epochs=args.epochs,
                        num_workers=args.workers, mcts_threads=args.mcts_threads, eval_games=args.arena_games,
                        batch_size=args.batch_size, lr=args.lr, eval_symmetry=args.eval_symmetry,
-                       full_search_prob=args.full_search_prob, fast_simulations=args.fast_simulations)
+                       full_search_prob=args.full_search_prob, fast_simulations=args.fast_simulations,
+                       arena_opening_plies=args.arena_opening_plies)
         if args.file_loop:
             az.run()                                                     # the reference's loop: data files between the stages
         else:

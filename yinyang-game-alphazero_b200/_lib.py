@@ -166,6 +166,7 @@ SIGNATURES = {
     "yy_selfplay_set_quota": (_I, [_P, _I64]),
     "yy_selfplay_set_random_stream": (_I, [_P, _P, _P, ctypes.c_int32, ctypes.c_int32]),
     "yy_selfplay_set_playout_cap": (_I, [_P, ctypes.c_double, ctypes.c_int32]),
+    "yy_arena_run": (_I, [_P, _P, _I64, _P, _P, _P, _P, ctypes.c_int32, _P, _P, _P]),
     "yy_selfplay_get_stats": (_I, [_P, ctypes.POINTER(SelfPlayStats), _P]),
     "yy_selfplay_replay": (_I, [_P, ctypes.POINTER(ReplayView)]),
     "yy_selfplay_stats_dev": (_P, [_P]),

@@ -41,11 +41,14 @@ def _barrier():
 class AlphaZero:
     def __init__(self, game, model_dir="models", data_dir="data", num_iterations=100, num_episodes=100, num_simulations=800,
                  num_epochs=10, temperature_threshold=10, update_threshold=0.6, num_workers=1, mcts_threads=1, eval_games=40,
-                 batch_size=64, lr=0.001, eval_symmetry="none", full_search_prob=1.0, fast_simulations=None):
+                 batch_size=64, lr=0.001, eval_symmetry="none", full_search_prob=1.0, fast_simulations=None,
+                 arena_opening_plies=0):
         self.game, self.model_dir, self.data_dir = game, model_dir, data_dir
         self.eval_symmetry = eval_symmetry      # leaf evaluation of the self-play and arena searches (Engine(eval_symmetry=))
         # playout cap randomisation of self-play (RollingSelfPlay); the arena always searches with num_simulations
         self.full_search_prob, self.fast_simulations = full_search_prob, fast_simulations
+        self.arena_opening_plies = arena_opening_plies     # > 0: arena games start from paired random openings
+        self._arena_round = 0                             # seeds the openings: every evaluation plays fresh ones
         self.num_iterations, self.num_episodes, self.num_simulations = num_iterations, num_episodes, num_simulations
         self.num_epochs, self.temperature_threshold, self.update_threshold = num_epochs, temperature_threshold, update_threshold
         self.num_workers, self.mcts_threads, self.eval_games = num_workers, mcts_threads, eval_games
@@ -82,8 +85,10 @@ class AlphaZero:
         return self.current_model_path
 
     def evaluate(self, current_model_path, best_model_path, num_games=None):  # alphazero.py:136-226
+        self._arena_round += 1
         return arena.evaluate(self.game, current_model_path, best_model_path, num_games=num_games or self.eval_games,
-                              num_simulations=self.num_simulations, mcts_threads=self.mcts_threads, eval_symmetry=self.eval_symmetry)
+                              num_simulations=self.num_simulations, mcts_threads=self.mcts_threads, eval_symmetry=self.eval_symmetry,
+                              opening_plies=self.arena_opening_plies, seed=self._arena_round)
 
     def update_best_model(self, win_ratio):  # alphazero.py:228-246
         if arena.should_promote(win_ratio, self.update_threshold):
@@ -108,7 +113,8 @@ class AlphaZero:
                           update_threshold=self.update_threshold, eval_games=self.eval_games, num_channels=C, num_res_blocks=B,
                           slots=slots, temperature_threshold=self.temperature_threshold, exact_episodes=exact_episodes,
                           mcts_threads=self.mcts_threads, state_dict=sd, eval_symmetry=self.eval_symmetry,
-                          full_search_prob=self.full_search_prob, fast_simulations=self.fast_simulations)
+                          full_search_prob=self.full_search_prob, fast_simulations=self.fast_simulations,
+                          arena_opening_plies=self.arena_opening_plies)
         try:
             return loop.run()
         finally:

@@ -68,6 +68,13 @@ struct EngineDev {
   int32_t* sp_moves_left;   // moves the slot may still make in this launch (INT_MAX = unlimited)
   long long game_quota;     // games that may be started in total since the last reset; < 0 = unlimited
   int32_t* act_list;        // [n_games] per CTA run: the games with a pending leaf, compacted, for the current iteration
+  // arena (yy_arena_run): n_games = 2G slots, slot j searches for model A and slot G + j for model B in arena game j.
+  // Game j keeps its board, player to move and ply in self-play slot j (sp_black, sp_white, sp_player, sp_step); sp_phase[s]
+  // = 1 while slot s has a search of the game in progress.
+  int32_t* ar_turn;         // [G] slot whose model is to move in game j, -1 once the game is over (the hand-off flag)
+  int8_t* ar_code;          // [G] YY_RESULT_* after the last move (player to move's view), 0 if the ply cap ended the game
+  uint8_t* ar_a_black;      // [G] 1 = model A plays black in game j
+  int ar_max_plies;         // a game that reaches this many plies ends with code 0
   // recorded random stream (test seam; replaces the np.random.choice / np.random.dirichlet draws of self_play.py:143-160
   // and mcts.py:303-306): uniforms [hook_games][hook_plies], Dirichlet samples [hook_games][A]; nullptr = Philox
   const double* hook_uniform; const double* hook_noise; int hook_games, hook_plies;

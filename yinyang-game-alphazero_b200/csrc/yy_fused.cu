@@ -35,11 +35,16 @@ struct FusedArgs {
   const uint64_t* black; const uint64_t* white;   // [count][W] boards to evaluate (search: the leaf batch)
   long long count;
   int boards_per_cta;          // contiguous run of boards (= games in a search) owned by a CTA
+  // arena: the grid is two halves of whole CTA pairs; CTAs [half_grid, grid) own boards [half_count, count) and stream the
+  // weight image at byte offset wb_off from the one above (same layout).  Other modes: half_grid = grid, half_count = count.
+  int half_grid;
+  long long half_count;
+  long long wb_off;
   int batch_boards;            // <= FC_N boards per heads pass (whole groups of g.Gb boards, except possibly the last group)
   __nv_bfloat16* headfeat;     // [count][64*A] head-conv features, index c*A + cell (L2-resident round trip)
   float* policy; float* value; float* logits;     // [count][A], [count], optional [count][A]
   int iterations;              // 1 = plain forward; n_sims + 1 = whole search; rolling self-play: any number of steps
-  int mode;                    // YY_FUSED_FORWARD / YY_FUSED_SEARCH (tree step after every evaluation) / YY_FUSED_SELFPLAY
+  int mode;                    // YY_FUSED_FORWARD / YY_FUSED_SEARCH (tree step after every evaluation) / YY_FUSED_SELFPLAY / YY_FUSED_ARENA
   int use_nn;                  // 0 = deterministic-prior (stub) evaluator: tree steps only
   int no_skew;                 // developer A/B (yy_engine_set_debug_flags bit 1): tiles of a group in lock step as in round 1
   int split_halves;            // developer A/B (yy_engine_set_debug_flags bit 0): the two halves of a group ping-pong through the
@@ -123,9 +128,13 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
   // of Gb boards.  In a pair both CTAs must walk the same batches / groups / tiles: the structure comes from the larger of
   // the two counts; entries past a CTA's own count are padding.
   auto clampl = [](long long v, long long hi) { return v < 0 ? 0 : (v > hi ? hi : v); };
-  const long long run_lo = (long long)blockIdx.x * a.boards_per_cta;
-  const int my_len = (int)clampl(a.count - run_lo, a.boards_per_cta);
-  const int st_len = (int)clampl(a.count - (long long)(blockIdx.x - rank) * a.boards_per_cta, a.boards_per_cta);
+  // (arena: both CTAs of a pair are in the same half, so they stream the same image and share the structural length)
+  const int half = (int)blockIdx.x >= a.half_grid ? 1 : 0, cta = (int)blockIdx.x - half * a.half_grid;
+  const long long run_lo = half * a.half_count + (long long)cta * a.boards_per_cta;
+  const int my_len = (int)clampl(a.half_count - (long long)cta * a.boards_per_cta, a.boards_per_cta);
+  const int st_len = (int)clampl(a.half_count - (long long)(cta - rank) * a.boards_per_cta, a.boards_per_cta);
+  const long long wofs = half ? a.wb_off : 0;    // weight image of this CTA pair: byte offset from image A
+  auto wf = [&](const float* p) { return reinterpret_cast<const float*>(reinterpret_cast<const uint8_t*>(p) + wofs); };
   const bool dyn = a.mode != YY_FUSED_FORWARD;
   volatile int* cnt_s = reinterpret_cast<volatile int*>(smem + SM_CNT);   // [step parity][cluster rank][leaves, selecting]
   const int E = a.n_avg;                         // walk entries per board (1 unless forms are averaged)
@@ -230,7 +239,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
             for (int l = 0; l < L; ++l) {
               const LayerInfo li = layer_info(l, g.blocks, CG);
               const uint32_t bytes = (uint32_t)li.stage_bytes / CG;     // pair: my half of the stage's output channels
-              const uint8_t* src = a.conv_stream + li.stream_off + (long long)rank * bytes;
+              const uint8_t* src = a.conv_stream + wofs + li.stream_off + (long long)rank * bytes;
               if (skew) {
 #pragma unroll
                 for (int t = 0; t < TW_MAXT; ++t) if (t < T) ++acc_nt[t];
@@ -253,7 +262,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
             mbar_wait(acc_full(0), (acc_n[0] - 1) & 1u);
             if (nh == 2) mbar_wait(acc_full(1), (acc_n[1] - 1) & 1u);
           }
-          const uint8_t* src = a.fc_stream;
+          const uint8_t* src = a.fc_stream + wofs;
           uint32_t fi = 0;
           fc_before = true;
           for (int h = 0; h < 2; ++h)
@@ -494,7 +503,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
           const int gi = sel[-k];
           do {      // at least one simulation per game and step: a search of S simulations ends within 2 (S + 1) steps
             const int np = tree_step_game<NW>(e, geo, gi, lane, nullptr, 1);
-            if (np == 0 && a.mode == YY_FUSED_SELFPLAY) sp_advance_game<NW>(e, geo, gi, lane);
+            if (np == 0 && a.mode >= YY_FUSED_SELFPLAY) advance_game<NW>(e, geo, gi, lane, a.mode);
             if (np != -1) break;
           } while (*stop != iter + 1);
         }
@@ -567,10 +576,11 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
       }
     };
     if (dyn) {
-      // self-play: slots without a search in progress (after a reset, or stopped on their move budget) get their next root
-      if (a.mode == YY_FUSED_SELFPLAY)
+      // self-play: slots without a search in progress (after a reset, or stopped on their move budget) get their next root;
+      // arena: a slot whose model the turn flag names (set by the other half of the grid) roots its search
+      if (a.mode >= YY_FUSED_SELFPLAY)
         for (int b = ew; b < my_len; b += TW_EPI_WARPS)
-          if (e.g_npending[run_lo + b] == 0) sp_advance_game<NW>(e, geo, (int)(run_lo + b), lane);
+          if (e.g_npending[run_lo + b] == 0) advance_game<NW>(e, geo, (int)(run_lo + b), lane, a.mode);
       epi_sync();
       compact(0);
     }
@@ -580,7 +590,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
       for (int k = ew; k < n_sel; k += TW_EPI_WARPS) {
         const int gi = my_list[my_len - 1 - k];
         const int np = tree_step_game<NW>(e, geo, gi, lane, nullptr, e.max_descents);
-        if (np == 0 && a.mode == YY_FUSED_SELFPLAY) sp_advance_game<NW>(e, geo, gi, lane);
+        if (np == 0 && a.mode >= YY_FUSED_SELFPLAY) advance_game<NW>(e, geo, gi, lane, a.mode);
       }
     };
     unsigned long long evals_here = 0;
@@ -718,7 +728,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
                 const uint32_t ready = CG == 2 ? mapa_u32(act_ready_t(t), 0) : act_ready_t(t);
                 auto arrive_t = [&]() { if (CG == 2) mbar_arrive_cluster(ready); else mbar_arrive(ready); };
                 stem_rows(t);
-                bias_t[tl] = __ldg(a.conv_bias + tl);                      // stem biases (buffer 0)
+                bias_t[tl] = __ldg(wf(a.conv_bias) + tl);                      // stem biases (buffer 0)
                 tc_fence_before();
                 fence_proxy_async_smem();
                 arrive_t();
@@ -727,7 +737,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
                   acct_phase ^= 1u << t;
                   tc_fence_after();
                   tile_sync();           // this layer's biases are staged by all four warps; the other buffer is free
-                  if (l + 1 < L) bias_t[((l + 1) & 1) * TW_C + tl] = __ldg(a.conv_bias + (size_t)(l + 1) * TW_C + tl);
+                  if (l + 1 < L) bias_t[((l + 1) & 1) * TW_C + tl] = __ldg(wf(a.conv_bias) + (size_t)(l + 1) * TW_C + tl);
                   layer_rows(l, t, 0, TW_C / 16, bias_t + (l & 1) * TW_C);
                   tc_fence_before();
                   if (l + 1 < L) {
@@ -746,7 +756,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
               fence_proxy_async_smem();
               arrive_act(hh);
             }
-            if (etid < TW_C) bias_s[etid] = __ldg(a.conv_bias + etid);     // stem biases (buffer 0)
+            if (etid < TW_C) bias_s[etid] = __ldg(wf(a.conv_bias) + etid);     // stem biases (buffer 0)
 
             for (int l = 0; l < L; ++l) {
               const bool is_head = (l == L - 1);
@@ -763,7 +773,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
                   arrive_act(hh);
                 }
               }
-              if (!is_head && etid < TW_C) bias_s[((l + 1) & 1) * TW_C + etid] = __ldg(a.conv_bias + (size_t)(l + 1) * TW_C + etid);
+              if (!is_head && etid < TW_C) bias_s[((l + 1) & 1) * TW_C + etid] = __ldg(wf(a.conv_bias) + (size_t)(l + 1) * TW_C + etid);
             }
           }
 
@@ -801,13 +811,13 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
             if (tile0 < fc.Tp) {
               const int o = tile0 * 128 + row;
               if (o < g.A) {
-                const float bo = __ldg(a.fc_policy_b + o);
+                const float bo = __ldg(wf(a.fc_policy_b) + o);
 #pragma unroll
                 for (int b = 0; b < 16; ++b) { sc_logit[b * 256 + o] = __uint_as_float(r0[b]) + bo; sc_logit[(b + 16) * 256 + o] = __uint_as_float(r1[b]) + bo; }
               }
             } else {
               const int o = (tile0 - fc.Tp) * 128 + row;
-              const float b1 = __ldg(a.fc_value1_b + o), w2 = __ldg(a.fc_value2_w + o);
+              const float b1 = __ldg(wf(a.fc_value1_b) + o), w2 = __ldg(wf(a.fc_value2_w) + o);
 #pragma unroll
               for (int b = 0; b < 16; ++b) {
                 sc_hidden[b * 256 + o] = fmaxf(__uint_as_float(r0[b]) + b1, 0.0f) * w2;
@@ -854,7 +864,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
               float acc = 0.0f;
               for (int k = lane; k < 256; k += 32) acc += sc_hidden[b * 256 + k];
               for (int off = 16; off; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
-              const float v = tanhf(acc + __ldg(a.fc_value2_b));
+              const float v = tanhf(acc + __ldg(wf(a.fc_value2_b)));
               if (E == 1) { if (lane == 0) a.value[board] = v; }
               else vsum += v;
               __syncwarp();
@@ -865,7 +875,8 @@ __global__ void __launch_bounds__(TW_THREADS, 1) fused_kernel(const FusedArgs a,
           if (dyn) {
             const int np = tree_step_game<NW>(e, geo, (int)board, lane, nullptr, e.max_descents);
             // search complete: the game makes its move and roots its next search now (self_play.py:139-190, :91-137)
-            if (np == 0 && a.mode == YY_FUSED_SELFPLAY) sp_advance_game<NW>(e, geo, (int)board, lane);
+            // (arena: the game makes its move and hands the turn to the other model's slot)
+            if (np == 0 && a.mode >= YY_FUSED_SELFPLAY) advance_game<NW>(e, geo, (int)board, lane, a.mode);
           }
         }
         phase(2);
@@ -916,9 +927,10 @@ static int launch_fused(NNState& nn, const FusedArgs& fa, const EngineDev& dev, 
 // Runs `iterations` evaluation (+ tree) steps over boards [0, count) in ONE launch.
 //   dev == nullptr : plain forward (do_tree off); policy/value/logits are the caller's output arrays.
 //   dev != nullptr : whole search over dev->leaf_* / eval_* (slot = game; leaves_per_step must be 1).
+//   YY_FUSED_ARENA : boards [count/2, count) are evaluated with the image `weights_b` (same geometry as the loaded one).
 int nn_fused_run(NNState& nn, const EngineDev* dev, uint32_t rule_flags, const uint64_t* black, const uint64_t* white, int64_t count,
                  float* policy, float* value, float* logits, int iterations, bool use_nn, int mode, const FormSpec& forms,
-                 cudaStream_t s) {
+                 cudaStream_t s, const void* weights_b) {
   if (use_nn) {
     if (!nn.attrs_set) return set_error(YY_ERR_STATE, "engine was not created with the NN evaluator");
     if (!nn.weights) return set_error(YY_ERR_STATE, "no weights loaded (yy_engine_load_weights)");
@@ -933,6 +945,8 @@ int nn_fused_run(NNState& nn, const EngineDev* dev, uint32_t rule_flags, const u
     return set_error(YY_ERR_INVALID, "fused run: %lld boards x %d forms exceed the head-feature scratch (%d boards, %d entries)",
                      (long long)count, E, nn.max_boards, nn.max_entries);
   if ((mode != YY_FUSED_FORWARD) != (dev != nullptr)) return set_error(YY_ERR_INVALID, "fused run: mode / engine state mismatch");
+  const bool arena = mode == YY_FUSED_ARENA;
+  if (arena && (!use_nn || !weights_b || (count & 1))) return set_error(YY_ERR_INVALID, "fused arena run: two images, an even count");
   FusedArgs fa{};
   fa.g = make_fused_geo(nn.rows, nn.cols, nn.blocks);
   fa.fc = make_fc_geo(nn.A);
@@ -966,6 +980,17 @@ int nn_fused_run(NNState& nn, const EngineDev* dev, uint32_t rule_flags, const u
   fa.boards_per_cta = (int)per;
   int grid = (int)((count + per - 1) / per);
   grid = (grid + 1) & ~1;                // whole CTA pairs; a trailing follower without boards only mirrors its leader's walk
+  fa.half_grid = grid; fa.half_count = count;
+  if (arena) {                           // each half of the grid gets whole CTA pairs over one model's boards
+    const long long half = count / 2;
+    per = (half + sms / 2 - 1) / (sms / 2);
+    if (per < 1) per = 1;
+    fa.boards_per_cta = (int)per;
+    fa.half_grid = ((int)((half + per - 1) / per) + 1) & ~1;
+    fa.half_count = half;
+    fa.wb_off = (long long)((uintptr_t)weights_b - (uintptr_t)nn.weights);
+    grid = 2 * fa.half_grid;
+  }
   EngineDev d{};
   if (dev) d = *dev;
   if (nn.profiling) {

@@ -39,8 +39,10 @@ struct EngineDev;
 //   YY_FUSED_SEARCH   whole search over the engine's leaf batch (slot = game); ends when no game has a pending leaf.
 //   YY_FUSED_SELFPLAY rolling self-play: a game whose search is complete makes its move and roots its next search in
 //                     the same step (sp_advance_game), within its move budget and the game quota.
+//   YY_FUSED_ARENA    two models in one launch (yy_arena_run): games [0, count/2) search with the loaded image, games
+//                     [count/2, count) with `weights_b`; a search that completes makes its arena move (arena_advance_game).
 // use_nn = false runs the deterministic-prior evaluator (tree steps only).
-enum { YY_FUSED_FORWARD = 0, YY_FUSED_SEARCH = 1, YY_FUSED_SELFPLAY = 2 };
+enum { YY_FUSED_FORWARD = 0, YY_FUSED_SEARCH = 1, YY_FUSED_SELFPLAY = 2, YY_FUSED_ARENA = 3 };
 // Symmetric evaluation: the dihedral form (form_src, yy_rules.cuh) the network sees a board in.
 //   IDENTITY  the board as it is;  FIXED  form `form` for every board;  HASHED  form hashed_form(stub_key(board), seed);
 //   AVERAGE   every valid form, policy and value averaged over them (fp32, ascending form order; no logits).
@@ -54,6 +56,6 @@ struct FormSpec {
 inline int form_entries(int mode, int rows, int cols) { return mode == YY_FORM_AVERAGE ? form_count(rows, cols) : 1; }
 int nn_fused_run(NNState& nn, const EngineDev* dev, uint32_t rule_flags, const uint64_t* black, const uint64_t* white,
                  int64_t count, float* policy, float* value, float* logits, int iterations, bool use_nn, int mode,
-                 const FormSpec& forms, cudaStream_t stream);
+                 const FormSpec& forms, cudaStream_t stream, const void* weights_b = nullptr);
 
 }  // namespace yy

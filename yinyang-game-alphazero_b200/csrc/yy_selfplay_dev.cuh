@@ -3,6 +3,7 @@
 // lock-step kernels of yy_tree.cu, lane 0 of the game's warp inside the persistent kernel of yy_fused.cu);
 // tree_root_game and sp_advance_game are executed by the whole warp that owns the game.
 #pragma once
+#include "yy_nn.cuh"
 #include "yy_tree_dev.cuh"
 
 namespace yy {
@@ -175,10 +176,9 @@ __device__ __forceinline__ void tree_root_game(const EngineDev& e, const Geo<NW>
 // Rolling self-play: called by the game's warp when the slot has no pending leaf -- either its search has just been
 // completed (make the move: sp_move_one) or the slot is waiting for its next root (after a reset, or after a launch
 // that ended on its move budget).  Leaves the slot with the root of its next search published as the pending leaf, or
-// idle (no budget / no game left in the quota).  Not inlined, arguments by value: the rare path keeps its registers and
-// its code out of the persistent kernel's hot loops, and the kernel's parameter structs stay in constant memory.
+// idle (no budget / no game left in the quota).
 template <int NW>
-__device__ __noinline__ void sp_advance_game(const EngineDev e, const Geo<NW> g, int gi, int lane) {
+__device__ __forceinline__ void sp_advance_game(const EngineDev& e, const Geo<NW>& g, int gi, int lane) {
   int budget = -1;
   if (lane == 0) {
     int left = e.sp_moves_left[gi];
@@ -198,6 +198,90 @@ __device__ __noinline__ void sp_advance_game(const EngineDev e, const Geo<NW> g,
   tree_root_game<NW>(e, g, gi, lane, budget);
   if (lane == 0) e.sp_phase[gi] = 1;
   __syncwarp();
+}
+
+// ------------------------------------------------------------------------------------------------ arena
+__device__ __forceinline__ int ld_acquire_gpu(const int32_t* p) {
+  int v;
+  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+
+// The slot of arena game j whose model moves for `player` (model A plays black iff ar_a_black[j]).
+__device__ __forceinline__ int arena_mover_slot(const EngineDev& e, int j, int player) {
+  return ((player == 1) == (e.ar_a_black[j] != 0)) ? j : (e.n_games >> 1) + j;
+}
+
+// One move of arena game j after slot s's search (AlphaZero.evaluate, alphazero.py:190-205, as arena.play_match plays it):
+// select_action(temperature = 0) = argmax of the root visit counts, lowest action on ties (no children / no visits:
+// action 0); getNextState with the mover's real player (an illegal action is a silent no-op, the turn passes); the game
+// ends on a nonzero getGameEnded for the next player or at the ply cap.  Otherwise the turn flag names the other model's
+// slot -- after the new state is visible device-wide: that slot lives in the other half of the grid.
+template <int NW>
+__device__ __forceinline__ void arena_move_one(const EngineDev& e, const Geo<NW>& g, int s, int j) {
+  const long long nb = (long long)s * e.max_nodes, eb = (long long)s * e.edges_cap;
+  const int base = e.node_edge_base[nb], cnt = (e.node_flags[nb] & NODE_EXPANDED) ? e.node_n_edges[nb] : 0;
+  int action = 0, best = 0;
+  for (int k = 0; k < cnt; ++k) {                       // children in ascending action order: strict '>' keeps the lowest
+    const int n = e.edge_N[eb + base + k];
+    if (n > best) { best = n; action = e.edge_action[eb + base + k]; }
+  }
+  BB<NW> b = load_bb<NW>(e.sp_black, j, e.W), w = load_bb<NW>(e.sp_white, j, e.W);
+  int player = e.sp_player[j];
+  apply_action(g, b, w, player, action);
+  player = -player;
+  const int ply = e.sp_step[j] + 1;
+  store_bb<NW>(e.sp_black, j, e.W, b); store_bb<NW>(e.sp_white, j, e.W, w);
+  e.sp_player[j] = (int8_t)player; e.sp_step[j] = ply;
+  atomicAdd(&e.stats->moves, 1ull);
+  const int code = ended_code(g, b, w, player);
+  if (code != 0 || ply >= e.ar_max_plies) {
+    e.ar_code[j] = (int8_t)code;
+    e.ar_turn[j] = -1;
+    atomicAdd(&e.stats->games_finished, 1ull);
+    return;
+  }
+  __threadfence();
+  *reinterpret_cast<volatile int32_t*>(e.ar_turn + j) = arena_mover_slot(e, j, player);
+}
+
+// Arena driver of slot s, the counterpart of sp_advance_game: called by the slot's warp when it has no search in progress.
+// A search that has just completed makes its move; then, if the turn flag names this slot, the slot roots a search of
+// the game for the player to move (no noise, n_sims simulations).  Nothing waits: a slot whose game is with the other
+// model stays idle, and a launch in which no slot of a CTA pair has work ends for that pair; the next launch's
+// start-of-launch pass picks the hand-off up.
+template <int NW>
+__device__ __forceinline__ void arena_advance_game(const EngineDev& e, const Geo<NW>& g, int s, int lane) {
+  int root = 0;
+  if (lane == 0) {
+    const int G = e.n_games >> 1, j = s < G ? s : s - G;
+    if (e.sp_phase[s]) {
+      e.sp_phase[s] = 0;
+      arena_move_one<NW>(e, g, s, j);
+    }
+    if (ld_acquire_gpu(e.ar_turn + j) == s) {
+      const BB<NW> b = load_bb<NW>(e.sp_black, j, e.W), w = load_bb<NW>(e.sp_white, j, e.W);
+      store_bb<NW>(e.root_black, s, e.W, b); store_bb<NW>(e.root_white, s, e.W, w);
+      e.root_player[s] = e.sp_player[j];
+      e.noise_mask[s] = 0;
+      root = 1;
+    }
+  }
+  root = __shfl_sync(kFull, root, 0);
+  if (!root) return;
+  __syncwarp();
+  tree_root_game<NW>(e, g, s, lane, e.n_sims);
+  if (lane == 0) e.sp_phase[s] = 1;
+  __syncwarp();
+}
+
+// The persistent kernel's driver of a slot without a search in progress (fused mode YY_FUSED_SELFPLAY: rolling self-play,
+// YY_FUSED_ARENA: the arena).  Not inlined, arguments by value: the rare path keeps its registers and its code out of the
+// persistent kernel's hot loops, and the kernel's parameter structs stay in constant memory.
+template <int NW>
+__device__ __noinline__ void advance_game(const EngineDev e, const Geo<NW> g, int gi, int lane, int mode) {
+  if (mode == YY_FUSED_ARENA) arena_advance_game<NW>(e, g, gi, lane);
+  else sp_advance_game<NW>(e, g, gi, lane);
 }
 
 }  // namespace yy

@@ -109,6 +109,31 @@ __global__ void sp_reset_kernel(EngineDev e) {
   for (int k = 0; k < e.W; ++k) { e.sp_black[(long long)gi * e.W + k] = 0; e.sp_white[(long long)gi * e.W + k] = 0; }
 }
 
+// ------------------------------------------------------------------------------------------------ arena
+// Start of arena game j (one thread per game): its start position goes to self-play slot j and the turn flag to the slot
+// of the model that moves first.  A start position that is already over ends the game with 0 plies.
+template <int NW>
+__global__ void arena_init_kernel(EngineDev e, Geo<NW> g, const uint64_t* black, const uint64_t* white, const int8_t* player,
+                                  const uint8_t* a_black) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= (e.n_games >> 1)) return;
+  const BB<NW> b = load_bb<NW>(black, j, e.W) & g.full, w = load_bb<NW>(white, j, e.W) & g.full;
+  const int p = player[j] == 1 ? 1 : -1;
+  store_bb<NW>(e.sp_black, j, e.W, b); store_bb<NW>(e.sp_white, j, e.W, w);
+  e.sp_player[j] = (int8_t)p; e.sp_step[j] = 0;
+  e.ar_a_black[j] = a_black[j] ? 1 : 0;
+  const int code = ended_code(g, b, w, p);
+  e.ar_code[j] = (int8_t)code;
+  e.ar_turn[j] = code != 0 ? -1 : arena_mover_slot(e, j, p);
+  if (code != 0) atomicAdd(&e.stats->games_finished, 1ull);
+}
+__global__ void arena_collect_kernel(EngineDev e, int8_t* code, int32_t* plies) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= (e.n_games >> 1)) return;
+  code[j] = e.ar_code[j];
+  plies[j] = e.sp_step[j];
+}
+
 // ------------------------------------------------------------------------------------------------ host side
 struct Carver {
   char* base; size_t off;
@@ -166,6 +191,7 @@ static void carve(const yy_engine_config& c, Carver& k, EngineDev& d) {
   d.sp_step = k.take<int32_t>(G); d.sp_passes = k.take<int32_t>(G); d.sp_serial = k.take<int32_t>(G);
   d.sp_new_game = k.take<uint8_t>(G); d.sp_full = k.take<uint8_t>(G); d.sp_next_serial = k.take<int32_t>(1);
   d.sp_phase = k.take<uint8_t>(G); d.sp_moves_left = k.take<int32_t>(G); d.act_list = k.take<int32_t>(G);
+  d.ar_turn = k.take<int32_t>(G); d.ar_code = k.take<int8_t>(G); d.ar_a_black = k.take<uint8_t>(G); d.ar_max_plies = 1;
   d.game_quota = -1; d.hook_uniform = nullptr; d.hook_noise = nullptr; d.hook_games = 0; d.hook_plies = 0;
   const size_t RC = (size_t)c.replay_capacity;
   d.replay_cap = (int)RC; d.results_cap = (int)(RC + G + 16);
@@ -523,6 +549,49 @@ int yy_selfplay_set_playout_cap(yy_engine* e, double full_prob, int32_t fast_sim
   e->dev.cap_threshold = (uint64_t)llround(full_prob * 4294967296.0);
   e->dev.fast_sims = fast_sims;
   return YY_OK;
+}
+
+int yy_arena_run(yy_engine* e, const void* weights_b, int64_t bytes, const uint64_t* start_black, const uint64_t* start_white,
+                 const int8_t* start_player, const uint8_t* a_plays_black, int32_t max_plies, int8_t* out_code, int32_t* out_plies,
+                 void* stream) {
+  if (!e) return set_error(YY_ERR_INVALID, "null engine");
+  if (e->cfg.evaluator != YY_EVAL_NN) return set_error(YY_ERR_STATE, "the arena needs the NN evaluator");
+  if (e->cfg.mode_flags & YY_MODE_STEP_KERNELS) return set_error(YY_ERR_STATE, "the arena runs on the persistent kernel, not YY_MODE_STEP_KERNELS");
+  if (e->cfg.leaves_per_step > 1) return set_error(YY_ERR_STATE, "the arena runs the exact search: leaves_per_step must be 1");
+  if (e->dev.n_games & 1) return set_error(YY_ERR_INVALID, "the arena needs an even n_games (two slots per game), not %d", e->dev.n_games);
+  const int64_t need = nn_weight_bytes(e->cfg.rows, e->cfg.cols, e->cfg.nn_channels, e->cfg.nn_blocks);
+  if (need < 0) return (int)need;
+  if (bytes != need) return set_error(YY_ERR_INVALID, "weight image B has %lld bytes, the engine's network needs %lld", (long long)bytes, (long long)need);
+  if (max_plies < 1) return set_error(YY_ERR_INVALID, "max_plies must be >= 1, not %d", (int)max_plies);
+  if (!weights_b || !start_black || !start_white || !start_player || !a_plays_black || !out_code || !out_plies)
+    return set_error(YY_ERR_INVALID, "null argument");
+  if (((uintptr_t)weights_b & 255) != 0) return set_error(YY_ERR_INVALID, "weight image B must be 256-byte aligned");
+  if (!e->nn.weights) return set_error(YY_ERR_STATE, "no weights loaded for model A (yy_engine_load_weights)");
+  cudaStream_t s = (cudaStream_t)stream;
+  const int G = e->dev.n_games / 2;
+  int rc = yy_selfplay_reset(e, stream); if (rc) return rc;
+  YY_DISPATCH_NW(e->dev.A, arena_init_kernel<NW><<<thread_grid(G, 128), 128, 0, s>>>(
+      e->dev, make_geo<NW>(e->cfg.rows, e->cfg.cols, e->cfg.rule_flags), start_black, start_white, start_player, a_plays_black));
+  YY_LAUNCH_CHECK();
+  EngineDev d = e->dev;
+  d.ar_max_plies = max_plies;
+  // a search needs at most 2 (n_sims + 1) evaluation steps, i.e. two launches, and the other model's slot picks the game up
+  // at the start of the next launch: every live game makes a move at least every two launches
+  const long long max_launches = 2ll * max_plies + 4;
+  for (long long launch = 0;; ++launch) {
+    Stats h;
+    YY_CUDA_OK(cudaMemcpyAsync(&h, e->dev.stats, sizeof(Stats), cudaMemcpyDeviceToHost, s));
+    YY_CUDA_OK(cudaStreamSynchronize(s));
+    if (h.overflow) return set_error(YY_ERR_CAPACITY, "a tree arena overflowed: raise edges_per_game");
+    if (h.games_finished >= (unsigned long long)G) break;
+    if (launch == max_launches) return set_error(YY_ERR_STATE, "arena: %d of %d games unfinished after %lld launches", G - (int)h.games_finished, G, launch);
+    rc = nn_fused_run(e->nn, &d, e->cfg.rule_flags, d.leaf_black, d.leaf_white, d.n_slots, d.eval_prior, d.eval_value, nullptr,
+                      e->cfg.n_sims + 1, true, YY_FUSED_ARENA, engine_forms(e), s, weights_b);
+    if (rc) return rc;
+  }
+  arena_collect_kernel<<<thread_grid(G, 128), 128, 0, s>>>(e->dev, out_code, out_plies);
+  YY_LAUNCH_CHECK();
+  return yy_selfplay_reset(e, stream);
 }
 
 int yy_selfplay_set_random_stream(yy_engine* e, const double* uniforms_dev, const double* noise_dev, int32_t n_games, int32_t n_plies) {

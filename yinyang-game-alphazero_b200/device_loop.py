@@ -127,12 +127,15 @@ class DeviceLoop:
     def __init__(self, game, model_dir="models", num_iterations=100, num_episodes=100, num_simulations=800, num_epochs=10,
                  batch_size=64, lr=0.001, weight_decay=1e-4, sample_size=10000, queue_size=500000, update_threshold=0.6, eval_games=40,
                  num_channels=128, num_res_blocks=10, slots=4096, temperature_threshold=10, exact_episodes=False, save_files=True,
-                 seed=0, mcts_threads=1, state_dict=None, eval_symmetry="none", full_search_prob=1.0, fast_simulations=None):
+                 seed=0, mcts_threads=1, state_dict=None, eval_symmetry="none", full_search_prob=1.0, fast_simulations=None,
+                 arena_opening_plies=0):
         self.game, self.model_dir = game, model_dir
         self.eval_symmetry = eval_symmetry
         self.num_iterations, self.num_episodes, self.num_simulations, self.num_epochs = num_iterations, num_episodes, num_simulations, num_epochs
         self.batch_size, self.sample_size, self.update_threshold, self.eval_games = batch_size, sample_size, update_threshold, eval_games
         self.exact_episodes, self.save_files, self.mcts_threads = exact_episodes, save_files, mcts_threads
+        self.seed, self.arena_opening_plies = seed, arena_opening_plies
+        self._device_arena = None
         self.dist, self.rank, self.world = _dist()
         n, m = game.getBoardSize()
         self.n, self.m = n, m
@@ -157,6 +160,8 @@ class DeviceLoop:
 
     def close(self):
         self.selfplay.close()
+        if self._device_arena is not None:
+            self._device_arena.close()
 
     # -- stages
     def _gather(self, rec):
@@ -193,8 +198,23 @@ class DeviceLoop:
             self.dist.broadcast(eng.weight_image, 0)
         eng.load_weight_image(eng.weight_image)
 
-    def _arena(self, current_sd):
-        """alphazero.py:136-226 on rank 0; every rank takes its verdict."""
+    def _arena(self, current_sd, it=0):
+        """alphazero.py:136-226.  mcts_threads = 1: the device arena (arena.DeviceArena) with the current weights against the
+        self-play engine's image of best_sd, the games sharded over the ranks in whole pairs and the counts all-reduced.
+        Otherwise rank 0 plays the host loop and every rank takes its verdict."""
+        from . import arena
+        if self.mcts_threads == 1 and self.eval_games > 0:
+            openings = arena.make_openings(self.game, self.eval_games, self.arena_opening_plies, self.seed * 1000003 + it)
+            C, B = _weights.infer_arch(current_sd)
+
+            def play(lo, hi):
+                if self._device_arena is None or self._device_arena.G != hi - lo:
+                    if self._device_arena is not None:
+                        self._device_arena.close()
+                    self._device_arena = arena.DeviceArena(self.game, hi - lo, self.num_simulations, C, B,
+                                                           eval_symmetry=self.eval_symmetry)
+                return self._device_arena.play(current_sd, self.selfplay.eng.weight_image, arena.shard_openings(openings, lo, hi))
+            return arena.play_sharded(self.eval_games, play, self.rank, self.world, device="cuda")["win_ratio"]
         ratio = 0.0
         if self.rank == 0 and self.eval_games > 0:
             from . import arena
@@ -231,7 +251,7 @@ class DeviceLoop:
         metrics, steps = self._train()
         sync(); t3 = time.perf_counter()
         current_sd = self.learner.state_dict()
-        ratio = self._arena(current_sd)
+        ratio = self._arena(current_sd, it)
         promoted = ratio >= self.update_threshold
         t4 = time.perf_counter()
         if promoted:

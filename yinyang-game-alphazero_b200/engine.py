@@ -285,6 +285,17 @@ def ended_host(boards, players, rows, cols, rule_flags=0):
 
 
 # ------------------------------------------------------------------------------------------------ engine
+def device_image(image, device):
+    """A packed weight image (numpy uint8, weights.pack_state_dict) -> a 256-byte aligned uint8 view on the device."""
+    with torch.cuda.device(device):
+        buf = torch.zeros(image.size + 256, dtype=torch.uint8, device=torch.device("cuda", device))
+        off = (-buf.data_ptr()) & 255
+        view = buf[off: off + image.size]
+        view.copy_(torch.from_numpy(image))
+        torch.cuda.synchronize()
+    return view
+
+
 @dataclass
 class Stats:
     moves: int
@@ -303,7 +314,8 @@ class Engine:
     def __init__(self, rows=8, cols=8, n_games=1, n_sims=800, evaluator="stub", cpuct=1.0, rule_flags=0,
                  search_as_black=True, edges_per_game=0, dirichlet_alpha=0.3, dirichlet_epsilon=0.25,
                  temperature_threshold=10, seed=0, replay_capacity=0, state_dict=None, nn_channels=128, nn_blocks=10,
-                 device=None, leaves_per_step=1, step_kernels=False, descents_per_step=0, eval_symmetry="none"):
+                 device=None, leaves_per_step=1, step_kernels=False, descents_per_step=0, eval_symmetry="none",
+                 weight_image=None):
         if eval_symmetry not in EVAL_SYMMETRY:
             raise ValueError(f"eval_symmetry must be one of {sorted(EVAL_SYMMETRY)}, not {eval_symmetry!r}")
         if eval_symmetry != "none" and evaluator != "nn":
@@ -319,7 +331,7 @@ class Engine:
         ev = {"stub": EVAL_STUB, "nn": EVAL_NN, "external": EVAL_EXTERNAL}[evaluator]
         self.evaluator = evaluator
         self.eval_symmetry = eval_symmetry
-        if evaluator == "nn":
+        if evaluator == "nn" and weight_image is None:      # (a packed image comes with nn_channels / nn_blocks)
             if state_dict is None:
                 raise ValueError("evaluator='nn' needs a reference state_dict / checkpoint dict")
             sd = state_dict["state_dict"] if "state_dict" in state_dict else state_dict
@@ -346,7 +358,9 @@ class Engine:
         if not self.handle:
             _lib.check(-1)
         self.weight_image = None
-        if evaluator == "nn":
+        if evaluator == "nn" and weight_image is not None:
+            self.load_weight_image(weight_image)
+        elif evaluator == "nn":
             self.load_state_dict(state_dict)
         self.replay_capacity = replay_capacity
         self.workspace_bytes = int(need)
@@ -367,13 +381,8 @@ class Engine:
     # -- weights (yy_engine_load_weights)
     def load_state_dict(self, state_dict):
         img = _weights.pack_state_dict(state_dict, self.rows, self.cols)
-        with torch.cuda.device(self.device):
-            buf = torch.zeros(img.size + 256, dtype=torch.uint8, device=self.tdev)
-            off = (-buf.data_ptr()) & 255
-            view = buf[off: off + img.size]
-            view.copy_(torch.from_numpy(img))
-            torch.cuda.synchronize()
-        self.weight_image, self._weight_buf = view, buf
+        view = device_image(img, self.device)
+        self.weight_image = view
         _lib.check(self.L.yy_engine_load_weights(self.handle, _ptr(view), img.size))
 
     def load_weight_image(self, image_u8: torch.Tensor):
@@ -550,6 +559,24 @@ class Engine:
         npl = int(u.shape[1]) if u is not None else (1 if z is not None else 0)
         self._random_stream = (u, z)                                   # the engine keeps the pointers: keep them alive
         _lib.check(self.L.yy_selfplay_set_random_stream(self.handle, _ptr(u), _ptr(z), ng, npl))
+
+    # -- arena (yy_arena_run)
+    def arena_run(self, image_b, start_black, start_white, start_player, a_plays_black, max_plies):
+        """n_games / 2 arena games, model A = the loaded weights (slots [0, G)), model B = image_b (a packed device image of
+        the same network shape, 256-byte aligned; slots [G, 2G)).  Device tensors in: start boards int64[G, W], players to
+        move int8[G], a_plays_black uint8/bool[G].  Every move is the temperature-0 choice of a noise-free search; a game
+        ends on a terminal position or after max_plies plies.  Returns device tensors (codes int8[G]: YY_RESULT_* of the
+        player to move after the last move, 0 at the ply cap; plies int32[G]).  Leaves the self-play slots reset."""
+        G = self.n_games // 2
+        _check_boards(start_black, start_white, start_player)
+        assert image_b.is_cuda and image_b.dtype == torch.uint8 and image_b.is_contiguous()
+        assert start_player.numel() == G and start_black.shape[0] == G and a_plays_black.numel() == G
+        ab = a_plays_black.to(device=self.tdev, dtype=torch.uint8).contiguous()
+        codes = torch.empty(G, dtype=torch.int8, device=self.tdev)
+        plies = torch.empty(G, dtype=torch.int32, device=self.tdev)
+        _lib.check(self.L.yy_arena_run(self.handle, _ptr(image_b), image_b.numel(), _ptr(start_black), _ptr(start_white),
+                                       _ptr(start_player), _ptr(ab), int(max_plies), _ptr(codes), _ptr(plies), _stream()))
+        return codes, plies
 
     def stats(self) -> Stats:
         s = _lib.SelfPlayStats()
